@@ -1,18 +1,18 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of Detect (decode + top-k + NMS) at 640x640, batch 64 per GPU (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode random|clustered]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mode random|clustered] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one Detect pass over one batch of B=64 synthetic head outputs per GPU (weak scaling: every rank owns its own
 64 images; for N>1 the step includes the gather of the fixed-shape detections block to rank 0, the only exchange the path
 has).  Prints ONE JSON line (rank 0).
 
-  value     frames/s, inputs resident in HBM: K steps issued back to back on ONE stream over 3 rotating input sets (165 MB per
-            GPU > 126 MB of L2) and `depth` rotating output buffers, timed on the device with one CUDA-event pair per block of
-            K steps, barrier + synchronize on both sides; the block is repeated (>= 5 times, >= 10 ms in total) and the MEDIAN
-            block is reported; max over ranks.  Consecutive calls overlap on the device (workspace ring, fdt_detect in
-            include/fdt_b200.h); completion stays in stream order.
+  value     frames/s, inputs resident in HBM: K = --steps steps issued back to back on ONE stream over 3 rotating input sets
+            (165 MB per GPU > 126 MB of L2) and `depth` rotating output buffers, after W = --warmup (at least 3) untimed steps
+            issued the same way; timed on the device with one CUDA-event pair around the K steps, barrier + synchronize on both
+            sides; max over ranks.  Consecutive calls overlap on the device (workspace ring, fdt_detect in include/fdt_b200.h);
+            completion stays in stream order.
   latency   the same step timed one at a time (own event pair, 256 MiB L2 flush + spin before it).
   e2e       frames/s through the public API with pinned HOST tensors: a stream of batches through Detect.submit(...).result()
             (fdt_detect_host_submit / _wait, two batches in flight; every batch's H2D copies, kernels and results inside the
@@ -25,6 +25,8 @@ has).  Prints ONE JSON line (rank 0).
             with a parity bit against the oracle, outside the headline timed region.
   gather_check (N>1) the fused gathered block on rank 0 == NCCL all-gather of every rank's local Detect output, byte for byte.
 --impl reference times the CPU port with all host threads as the reference arm.
+--dump-outputs DIR writes the detections block [B x N_GPUs, 2, top_k, 5] (float32) that the last timed step returned to
+DIR/detections.npy; the synthetic inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import glob
@@ -58,6 +60,9 @@ def parse():
     ap.add_argument("--mode", default="random", choices=["random", "clustered"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last timed step to DIR/<name>.npy (float32), "
+                         "to compare two builds output for output; the inputs depend on the arguments only")
     ap.add_argument("--depth", type=int, default=0, help="workspace slots (calls that may overlap on the device); 0 = library default")
     ap.add_argument("--gather", default="peer", choices=["peer", "peer-inline", "peer-barrier", "peer-all", "nccl"],
                     help="N>1: peer = rows stored into rank 0's gathered block by the NMS kernel over NVLink, completion signalled through "
@@ -112,6 +117,14 @@ def profile_summary():
     rel, d = os.path.relpath(best[0], ROOT), best[1]
     return {"traffic": float(d["dram_bytes_read"]) + float(d["dram_bytes_write"]), "traffic_source": rel + ": " + d.get("traffic_note", ""),
             "kernel_share_of_step": d.get("kernel_share_of_step"), "share_source": rel + ": " + d.get("share_note", "")}
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> float32 / float64 ndarray, written as out_dir/<name>.npy"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def host_threads():
@@ -207,8 +220,10 @@ def run_reference(args):
         det(loc, conf, pri)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        det(loc, conf, pri)
+        out = det(loc, conf, pri)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"detections": out})
     fps = args.steps * B_PER_GPU / dt
     line = {"impl": "reference", "metric": METRIC, "value": fps,
             "unit": "frames/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -443,42 +458,39 @@ def main():
         cur[0] += 1
 
     spin_cycles = 250_000
-    for _ in range(max(args.warmup, 3)):
-        flush.zero_()
-        torch.cuda._sleep(spin_cycles)
+    torch.cuda._sleep(spin_cycles)
+    for _ in range(max(args.warmup, 3)):                # untimed steps, issued back to back like the timed ones
         step()
     torch.cuda.synchronize()
 
     sampler = ClockSampler(local)
     sampler.start()
-    # ---- throughput: blocks of K steps back to back over the rotating input sets, one event pair per block, barrier + synchronize
-    #      on both sides of every block; the median block is reported
-    blocks_ms = []
+    # ---- throughput: the K = --steps timed steps back to back over the rotating input sets, one event pair around them, barrier +
+    #      synchronize on both sides
+    if world > 1:
+        dist.barrier()
+    torch.cuda.synchronize()
     wall0 = time.perf_counter()
     sampler.active = True
-    n_blocks = 0
-    while n_blocks < 5 or (sum(blocks_ms) < 10.0 and n_blocks < 50):
-        if world > 1:
-            dist.barrier()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        torch.cuda._sleep(2_000_000)                    # ~1 ms of GPU spin: the host gets ahead, the pair sees device time only
-        e0.record()
-        for i in range(args.steps):
-            step()
-        if peer is not None:
-            peer.wait_ready()                           # (await kernels on their own stream: the timed stream waits for the last one)
-        e1.record()
-        torch.cuda.synchronize()
-        if world > 1:
-            dist.barrier()
-        t = torch.tensor([float(e0.elapsed_time(e1))], dtype=torch.float64, device=dev)
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)    # every block: max over ranks
-        blocks_ms.append(float(t.item()))
-        n_blocks += 1
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda._sleep(2_000_000)                        # ~1 ms of GPU spin: the host gets ahead, the pair sees device time only
+    e0.record()
+    for _ in range(args.steps):
+        step()
+    if peer is not None:
+        peer.wait_ready()                               # (await kernels on their own stream: the timed stream waits for the last one)
+    e1.record()
+    torch.cuda.synchronize()
     wall = time.perf_counter() - wall0
-    total_ms = float(statistics.median(blocks_ms))
+    if world > 1:
+        dist.barrier()
+    t = torch.tensor([float(e0.elapsed_time(e1))], dtype=torch.float64, device=dev)
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)        # max over ranks
+    total_ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        # the detections block the last timed step returned (N > 1: rank 0's gathered block of every rank's images)
+        dump_outputs(args.dump_outputs, {"detections": last_block[0].cpu().numpy()})
     # ---- N>1: the gathered block the timed path produced must equal the NCCL all-gather of the ranks' local outputs
     gather_check = None
     if world > 1:
@@ -688,14 +700,14 @@ def main():
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": workload_config(args.mode, world),
             "l2": f"inputs larger than L2: {ROTATE} rotating input sets per GPU ({ROTATE * 54.9:.0f} MB > 126 MB), steps issued back to back on one stream",
-            "timing": {"blocks": n_blocks, "steps_per_block": args.steps, "block_ms": blocks_ms, "reported": "median block",
-                       "how": "one CUDA-event pair per block of K steps on the launching stream, barrier + synchronize on both sides of every block, "
-                              "max over ranks per block", "workspace_depth": depth,
+            "timing": {"steps": args.steps, "ms": total_ms,
+                       "how": "one CUDA-event pair around the K steps on the launching stream, barrier + synchronize on both sides, "
+                              "max over ranks", "workspace_depth": depth,
                        "overlap": "consecutive calls overlap on the device (workspace ring of `depth` slots; completion in stream order)"},
             "latency": {"ms_per_step": lat_ms, "frames_per_s": world * B / (lat_ms * 1e-3), "steps": n_lat,
                         "how": "each step alone with its own event pair; 256 MiB L2 flush + 0.1 ms GPU spin before it (outside the pair)"},
             "clocks": sampler.result(), "e2e": e2e,
-            "gpu_launches": launches_per_step * args.steps * n_blocks,      # k_detect_begin, k_sort_nms<fused> (+ k_gather_await on rank 0)
+            "gpu_launches": launches_per_step * args.steps,      # k_detect_begin, k_sort_nms<fused> (+ k_gather_await on rank 0)
             "gpu_launches_per_step": launches_per_step,
             "wall_s_timed_region": wall}
     if world > 1:
