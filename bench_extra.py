@@ -10,6 +10,7 @@
                                      # BASELINE config 5: Detect B=512 @1024^2 sharded over N GPUs, gather fused / NCCL
     python bench_extra.py torchref   # BASELINE.md 5.4: the reference's python-loop Detect restated in torch, on CUDA tensors and on the CPU
     python bench_extra.py heads      # SURVEY 8f rank 1: Detect straight from the per-level NCHW head maps, B=64 @640^2
+    python bench_extra.py heads_train # SURVEY 8f rank 1: MultiBoxLoss (+ backward) straight from the head maps, B=32 @640^2 (config 3)
 
 Each prints one JSON line with device time (CUDA events, L2 flushed between repetitions), the algorithmic bytes of
 SURVEY 8(d) and the CPU oracle port timed on the host beside it."""
@@ -402,6 +403,99 @@ def heads():
                       "torch_head_ops_then_detect_ms": ms_t, "torch_head_ops_ms": ms_th,
                       "algorithmic_bytes": alg, "roofline_frac_of_measured_hbm": alg / (ms_f * 1e-3) / 1e9 / PEAK,
                       "rows_kept_per_image": cand}))
+
+
+def heads_train():
+    """MultiBoxLoss from the per-level NCHW head maps, B=32 @640x640 (N=34,125), the ground truth of config 3, both matchers:
+    forward and forward+backward (gradients down to the maps) for (1) the reference's head ops restated in torch + the library's
+    MultiBoxLoss -- the only way to map gradients before fdt_multibox_loss_forward_heads --, (2) fdt_heads_to_loc_conf +
+    fdt_multibox_loss_forward (two steps, [B,N,4] / [B,N,2] materialised both ways) and (3) the fused entries."""
+    from fdt_b200.layers import MultiBoxLoss, heads_to_loc_conf
+    from fdt_b200.layers.functions.heads import _level_args
+    from fdt_b200.layers.modules.multibox_loss import pack_targets
+    from tests.torch_heads_ref import heads as torch_heads
+    B = 32
+    pri_np = synth.priors_numpy(640, 640); N = pri_np.shape[0]
+    loc_maps, conf_maps, neg_max = synth.head_maps(B, 640, 640, 3032)
+    _, _, targets = synth.multibox_inputs(B, pri_np, 3030, 0, 200)
+    dev = torch.device("cuda")
+    p = torch.from_numpy(pri_np).to(dev)
+    tg = [torch.from_numpy(t).to(dev) for t in targets]
+    lm, cm = [torch.from_numpy(m).to(dev) for m in loc_maps], [torch.from_numpy(m).to(dev) for m in conf_maps]
+    gt, off, G = pack_targets(tg, dev)
+    _, _, _, keep, (lp, cp, fh, fw, nm, nl) = _level_args(lm, cm, neg_max)
+    L = _lib.lib(); st = _lib.stream_ptr()
+    losses = torch.empty(2, device=dev); norm = torch.empty(1, device=dev)
+    loc_t = torch.empty((B, N, 4), device=dev); conf_t = torch.empty((B, N), dtype=torch.int64, device=dev)
+    sel = torch.empty((B, N), dtype=torch.uint8, device=dev)
+    loc_b = torch.empty((B, N, 4), device=dev); conf_b = torch.empty((B, N, 2), device=dev)
+    ws = _lib.workspace(L.fdt_multibox_workspace_bytes(B, N, 2, G), dev, "htx")
+
+    def leaves():
+        return [m.clone().requires_grad_(True) for m in lm], [m.clone().requires_grad_(True) for m in cm]
+    res = {}
+    for bip in (False, True):
+        crit = MultiBoxLoss(2, 0.35, True, 0, True, 3, 0.35, False, bipartite=bip)
+
+        def c_two_step():
+            _lib.check(L.fdt_heads_to_loc_conf(lp, cp, fh, fw, nm, nl, B, 0, loc_b.data_ptr(), conf_b.data_ptr(), st))
+            _lib.check(L.fdt_multibox_loss_forward(loc_b.data_ptr(), conf_b.data_ptr(), p.data_ptr(), gt.data_ptr(), off.data_ptr(), G, B, N, 2,
+                                                   0.35, 3, int(bip), 0.1, 0.2, losses.data_ptr(), norm.data_ptr(), loc_t.data_ptr(),
+                                                   conf_t.data_ptr(), sel.data_ptr(), None, ws.data_ptr(), ws.numel(), st))
+
+        def c_fused():
+            _lib.check(L.fdt_multibox_loss_forward_heads(lp, cp, fh, fw, nm, nl, p.data_ptr(), gt.data_ptr(), off.data_ptr(), G, B, 0.35, 3,
+                                                         int(bip), 0.1, 0.2, losses.data_ptr(), norm.data_ptr(), loc_t.data_ptr(),
+                                                         conf_t.data_ptr(), sel.data_ptr(), None, ws.data_ptr(), ws.numel(), st))
+        c_two_step(); torch.cuda.synchronize()
+        l2, ct2, s2 = losses.clone(), conf_t.clone(), sel.clone()
+        c_fused(); torch.cuda.synchronize()
+        fwd_parity = bool(torch.equal(ct2, conf_t) and torch.equal(s2, sel) and torch.allclose(l2, losses, rtol=1e-6, atol=0))
+
+        def torch_fwd():
+            with torch.no_grad():
+                crit((*torch_heads(lm, cm, neg_max, False), p), tg)
+
+        def fb(path):
+            lh, ch = leaves()
+
+            def run():
+                if path == "torch":
+                    ll, lc = crit((*torch_heads(lh, ch, neg_max, False), p), tg)
+                elif path == "two_step":
+                    ll, lc = crit((*heads_to_loc_conf(lh, ch, neg_max, softmax=False), p), tg)
+                else:
+                    ll, lc = crit.forward_heads(lh, ch, p, tg, neg_max)
+                (ll + lc).backward()
+                return ll, lc, [m.grad for m in lh + ch]
+            return run
+        outs = {k: fb(k)() for k in ("torch", "two_step", "fused")}
+        grads_bit_equal = all(torch.equal(a.view(torch.int32), b.view(torch.int32)) for a, b in zip(outs["two_step"][2], outs["fused"][2]))
+        torch_close = all(torch.allclose(a, b, rtol=1e-4, atol=1e-7) for a, b in zip(outs["torch"][2], outs["fused"][2])) and \
+            all(torch.allclose(outs["torch"][i], outs["fused"][i], rtol=1e-5) for i in (0, 1))
+        r = {"fwd_ms": {"torch_heads_plus_library_loss": timed(torch_fwd)[0], "two_step": timed(c_two_step)[0], "fused": timed(c_fused)[0]},
+             "fwd_bwd_ms": {k: timed(fb(k), reps=10)[0] for k in ("torch", "two_step", "fused")},
+             "parity": {"fused_fwd_equals_two_step": fwd_parity, "fused_map_grads_bit_equal_two_step": bool(grads_bit_equal),
+                        "torch_path_close": bool(torch_close)}}
+        r["fused_fwd_beats_two_step"] = r["fwd_ms"]["fused"] < r["fwd_ms"]["two_step"]
+        fwd_b = B * 56 * N + 20 * G                    # maps 32 B/prior read, loc_t + conf_t 24 B/prior written, GT rows
+        r["fused_fwd_gbs"] = fwd_b / (r["fwd_ms"]["fused"] * 1e-3) / 1e9
+        res["bipartite" if bip else "default"] = r
+    # backward alone, fused entry, default matcher (the forward above left loc_t / conf_t / sel / norm in place)
+    gmaps_l = [torch.empty_like(m) for m in lm]; gmaps_c = [torch.empty_like(m) for m in cm]
+    import ctypes as C
+    glp = (C.c_void_p * nl)(*[t.data_ptr() for t in gmaps_l]); gcp = (C.c_void_p * nl)(*[t.data_ptr() for t in gmaps_c])
+    one = torch.ones((), device=dev)
+
+    def c_bwd():
+        _lib.check(L.fdt_multibox_loss_backward_heads_dev(lp, cp, fh, fw, nm, nl, loc_t.data_ptr(), conf_t.data_ptr(), sel.data_ptr(),
+                                                          norm.data_ptr(), one.data_ptr(), one.data_ptr(), B, glp, gcp, st))
+    ms_bwd, _ = timed(c_bwd)
+    print(json.dumps({"workload": "MultiBoxLoss from per-level NCHW head maps, B=32 @640x640 (N=34,125), GT of config 3", "gt_total": G,
+                      "device": torch.cuda.get_device_name(), "results": res,
+                      "fused_fwd_algorithmic_bytes": B * 56 * N + 20 * G, "fused_bwd_algorithmic_bytes": B * 89 * N,
+                      "fused_bwd_ms": ms_bwd, "fused_bwd_gbs": B * 89 * N / (ms_bwd * 1e-3) / 1e9,
+                      "materialisation_removed_bytes": {"forward": B * 56 * N, "backward": B * 72 * N}}))
 
 
 if __name__ == "__main__":

@@ -5,8 +5,8 @@ pyramid_mobile_try1.py:297-327 and pyramid_mb2_try3/4/5.py): per pyramid level t
 reduced to (neg, pos) by max-in-out, both maps are permuted NCHW -> NHWC, flattened and concatenated over the
 levels into loc[B,N,4] / conf[B,N,2], and the test phase applies a 2-way softmax before Detect.
 
-`heads_to_loc_conf` materialises exactly those tensors with one kernel; `Detect.detect_heads` (detection.py here)
-skips the materialisation altogether.  No CPU fallback.
+`heads_to_loc_conf` materialises exactly those tensors with one kernel and is differentiable; `Detect.detect_heads`
+(detection.py here) and `MultiBoxLoss.forward_heads` (multibox_loss.py) skip the materialisation altogether.  No CPU fallback.
 """
 from __future__ import annotations
 
@@ -45,9 +45,58 @@ def _level_args(loc_maps, conf_maps, neg_max):
     return dev, B, N, (conf, loc), (lp, cp, fh, fw, nm, L)
 
 
+def _map_grads(maps, needed, dev):
+    """fp32 gradient buffers shaped like `maps` (None where not needed) and their ctypes pointer array (None if none is needed)."""
+    if not needed:
+        return None, None
+    g = [torch.empty(tuple(m.shape), dtype=torch.float32, device=dev) for m in maps]
+    return g, (C.c_void_p * len(g))(*[t.data_ptr() for t in g])
+
+
+class _HeadsToLocConfFn(torch.autograd.Function):
+    """heads_to_loc_conf with a backward: loc rows copied into the loc maps, conf rows (through the softmax's backward when it
+    was applied) routed into the conf maps the way torch's chunk / max / cat backward routes them."""
+
+    @staticmethod
+    def forward(ctx, neg_max, softmax, L, *maps):
+        loc_maps, conf_maps = maps[:L], maps[L:]
+        dev, B, N, (conf, loc), (lp, cp, fh, fw, nm, _) = _level_args(loc_maps, conf_maps, neg_max)
+        with torch.cuda.device(dev):
+            loc_out = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
+            conf_out = torch.empty((B, N, 2), dtype=torch.float32, device=dev)
+            _lib.check(_lib.lib().fdt_heads_to_loc_conf(lp, cp, fh, fw, nm, L, B, 1 if softmax else 0,
+                                                        _lib.ptr(loc_out), _lib.ptr(conf_out), _lib.stream_ptr()))
+        ctx.save_for_backward(*conf)
+        ctx.level = (fh, fw, nm, L, B, softmax, dev)
+        return loc_out, conf_out
+
+    @staticmethod
+    def backward(ctx, g_loc, g_conf):
+        conf = ctx.saved_tensors
+        fh, fw, nm, L, B, softmax, dev = ctx.level
+        need_loc, need_conf = any(ctx.needs_input_grad[3:3 + L]), any(ctx.needs_input_grad[3 + L:])
+        gl_maps, glp = _map_grads(conf, need_loc, dev)           # (loc maps have the conf maps' shape)
+        gc_maps, gcp = _map_grads(conf, need_conf, dev)
+        gl = _lib.dev_f32(g_loc, dev) if need_loc else None
+        gc = _lib.dev_f32(g_conf, dev) if need_conf else None
+        cp = (C.c_void_p * L)(*[m.data_ptr() for m in conf])
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().fdt_heads_to_loc_conf_backward(cp, fh, fw, nm, L, B, 1 if softmax else 0, _lib.ptr(gl), _lib.ptr(gc),
+                                                                 glp, gcp, _lib.stream_ptr()))
+        return (None, None, None, *(gl_maps or [None] * L), *(gc_maps or [None] * L))
+
+
 def heads_to_loc_conf(loc_maps, conf_maps, neg_max=None, softmax=True):
     """Per-level NCHW maps -> (loc[B,N,4], conf[B,N,2]) as pyramid.py:291-309 builds them; softmax=True also
-    applies nn.Softmax(dim=-1) (:332, test phase), softmax=False keeps the raw logits MultiBoxLoss consumes."""
+    applies nn.Softmax(dim=-1) (:332, test phase), softmax=False keeps the raw logits MultiBoxLoss consumes.
+    Differentiable: when a map requires grad, backward writes the gradients of the maps (those of the max-in-out
+    reduction go where torch's max(dim) backward sends them)."""
+    if torch.is_grad_enabled() and any(m.requires_grad for m in (*loc_maps, *conf_maps)):
+        L = len(conf_maps)
+        if len(loc_maps) != L:
+            raise ValueError("heads: need one loc map and one conf map per pyramid level")
+        nmx = None if neg_max is None else tuple(int(bool(v)) for v in neg_max)
+        return _HeadsToLocConfFn.apply(nmx, bool(softmax), L, *loc_maps, *conf_maps)
     dev, B, N, keep, (lp, cp, fh, fw, nm, L) = _level_args(loc_maps, conf_maps, neg_max)
     with torch.cuda.device(dev):
         loc = torch.empty((B, N, 4), dtype=torch.float32, device=dev)

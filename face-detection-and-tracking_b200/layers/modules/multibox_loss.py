@@ -1,11 +1,14 @@
 """MultiBoxLoss -- drop-in for layers/modules/multibox_loss.py:9-136 on hand-written sm_100a kernels."""
 from __future__ import annotations
 
+import ctypes as C
+
 import torch
 import torch.nn as nn
 
 from ... import _lib
 from ...data import face as cfg
+from ..functions.heads import _level_args, _map_grads
 
 
 def pack_targets(targets, device):
@@ -78,6 +81,54 @@ class _MultiBoxLossFn(torch.autograd.Function):
         return grad_loc, grad_conf, None, None, None, None, None, None, None, None
 
 
+class _MultiBoxLossHeadsFn(torch.autograd.Function):
+    """MultiBoxLoss straight from the per-level NCHW head maps (C = 2): the loss kernels read the maps, the backward writes
+    the map gradients -- nothing [B,N,4] / [B,N,2] is materialised in either direction."""
+
+    @staticmethod
+    def forward(ctx, priors, gt, gt_off, total_gt, threshold, negpos_ratio, bipartite, variance, neg_max, L, *maps):
+        dev, B, N, (conf, loc), (lp, cp, fh, fw, nm, _) = _level_args(maps[:L], maps[L:], neg_max)
+        pri = _lib.dev_f32(priors, dev)
+        if pri.dim() != 2 or pri.size(1) != 4 or pri.size(0) != N:
+            raise ValueError(f"MultiBoxLoss.forward_heads: priors must be [{N},4] (one per map position), got {tuple(pri.shape)}")
+        losses = torch.empty(2, dtype=torch.float32, device=dev)
+        norm = torch.empty(1, dtype=torch.float32, device=dev)
+        loc_t = torch.empty((B, N, 4), dtype=torch.float32, device=dev)
+        conf_t = torch.empty((B, N), dtype=torch.int64, device=dev)
+        sel = torch.empty((B, N), dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            lib = _lib.lib()
+            ws = _lib.workspace(lib.fdt_multibox_workspace_bytes(B, N, 2, total_gt), dev, "multibox")
+            _lib.check(lib.fdt_multibox_loss_forward_heads(
+                lp, cp, fh, fw, nm, L, _lib.ptr(pri), _lib.ptr(gt), _lib.ptr(gt_off), total_gt, B,
+                float(threshold), int(negpos_ratio), int(bool(bipartite)), float(variance[0]), float(variance[1]),
+                _lib.ptr(losses), _lib.ptr(norm), _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), None,
+                _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+        ctx.save_for_backward(loc_t, conf_t, sel, norm, *loc, *conf)
+        ctx.level = (fh, fw, nm, L, B, dev)
+        ctx.mark_non_differentiable(loc_t, conf_t, sel)
+        return losses[0].clone(), losses[1].clone(), loc_t, conf_t, sel
+
+    @staticmethod
+    def backward(ctx, g_l, g_c, *_):
+        fh, fw, nm, L, B, dev = ctx.level
+        loc_t, conf_t, sel, norm, *maps = ctx.saved_tensors
+        loc, conf = maps[:L], maps[L:]
+        need_loc, need_conf = any(ctx.needs_input_grad[10:10 + L]), any(ctx.needs_input_grad[10 + L:])
+        gl_maps, glp = _map_grads(loc, need_loc, dev)
+        gc_maps, gcp = _map_grads(conf, need_conf, dev)
+        zero = torch.zeros((), dtype=torch.float32, device=dev)
+        gl = zero if g_l is None else g_l.detach().to(device=dev, dtype=torch.float32).contiguous()
+        gc = zero if g_c is None else g_c.detach().to(device=dev, dtype=torch.float32).contiguous()
+        lp = (C.c_void_p * L)(*[m.data_ptr() for m in loc])
+        cp = (C.c_void_p * L)(*[m.data_ptr() for m in conf])
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().fdt_multibox_loss_backward_heads_dev(
+                lp, cp, fh, fw, nm, L, _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), _lib.ptr(norm),
+                _lib.ptr(gl), _lib.ptr(gc), B, glp, gcp, _lib.stream_ptr()))
+        return (None,) * 10 + (*(gl_maps or [None] * L), *(gc_maps or [None] * L))
+
+
 class MultiBoxLoss(nn.Module):
     """SSD weighted loss (multibox_loss.py:9-30): match + encode, smooth-L1 on positives, hard-negative
     mining (negpos_ratio:1), cross-entropy over positives and mined negatives, both divided by the
@@ -121,3 +172,24 @@ class MultiBoxLoss(nn.Module):
             self.variance)
         self.last_aux = (loc_t, conf_t, sel)
         return loss_l.to(src), loss_c.to(src)
+
+    def forward_heads(self, loc_maps, conf_maps, priors, targets, neg_max=None):
+        """The loss straight from the models' per-level NCHW head maps (pyramid.py:291-309): loc_maps[l] [B,4,H_l,W_l] and the
+        4-channel max-in-out conf_maps[l] [B,4,H_l,W_l]; neg_max[l] as in heads_to_loc_conf (default: level 0 reduces the
+        negatives).  Equals forward((*heads_to_loc_conf(loc_maps, conf_maps, neg_max, softmax=False), priors), targets), and is
+        differentiable with respect to every map that requires grad, without materialising loc / conf or their gradients."""
+        if self.num_classes != 2:
+            raise NotImplementedError("MultiBoxLoss.forward_heads: the head maps carry two classes (num_classes=2)")
+        L = len(conf_maps)
+        if len(loc_maps) != L:
+            raise ValueError("MultiBoxLoss.forward_heads: need one loc map and one conf map per pyramid level")
+        dev = _lib.require_cuda()
+        if conf_maps[0].is_cuda:
+            dev = conf_maps[0].device
+        gt, gt_off, total = pack_targets(targets, dev)
+        nmx = None if neg_max is None else tuple(int(bool(v)) for v in neg_max)
+        loss_l, loss_c, loc_t, conf_t, sel = _MultiBoxLossHeadsFn.apply(
+            priors, gt, gt_off, total, self.threshold, self.negpos_ratio, self.bipartite, self.variance, nmx, L,
+            *loc_maps, *conf_maps)
+        self.last_aux = (loc_t, conf_t, sel)
+        return loss_l, loss_c

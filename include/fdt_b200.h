@@ -318,6 +318,32 @@ int fdt_multibox_loss_backward_dev(const float *loc, const float *conf, const fl
                                    const uint8_t *sel, const float *norm, const float *g_l_dev, const float *g_c_dev,
                                    int B, int64_t N, int C, float *grad_loc, float *grad_conf, fdt_stream_t stream);
 
+/* ---- training from head maps (SURVEY 8f rank 1; replaces pyramid.py:291-309 + MyTrain_repo.py:170-171 and their autograd backward)
+ * Map arguments as fdt_heads_to_loc_conf (HOST arrays of n_levels DEVICE pointers, NCHW [B,4,H_l,W_l]); N = sum H_l*W_l, C = 2.
+ * Gradient maps have the maps' layout.  The gradient of a max-reduced logit goes to the channel torch's max(dim) backward picks: the
+ * first NaN of the three channels if there is one, else the lowest channel equal to their maximum (-0.0 == +0.0); the other two
+ * channels of the three receive +0.0.
+ * fdt_heads_to_loc_conf_backward: the backward of fdt_heads_to_loc_conf.  grad_loc[B,N,4] / grad_conf[B,N,2] may each be null, and
+ *   then the matching map gradients are not written (nor read: their array may be null); otherwise every element of them is written.
+ *   softmax != 0 applies the 2-way softmax's backward y * (g - (g0*y0 + g1*y1)) first, y recomputed from conf_maps_h.
+ * fdt_multibox_loss_forward_heads == fdt_heads_to_loc_conf(softmax = 0) + fdt_multibox_loss_forward(C = 2), with the same outputs
+ *   and nothing materialised: the kernels read the maps.  priors[N,4]; workspace fdt_multibox_workspace_bytes(B, N, 2, total_gt).
+ * fdt_multibox_loss_backward_heads_dev == fdt_multibox_loss_backward_dev + fdt_heads_to_loc_conf_backward(softmax = 0), bit-identical,
+ *   writing the map gradients directly (either gradient array may be null: not written).  Device scalars, graph capturable. */
+int fdt_heads_to_loc_conf_backward(const float *const *conf_maps_h, const int *f_h, const int *f_w, const int *neg_max_h,
+                                   int n_levels, int B, int softmax, const float *grad_loc, const float *grad_conf,
+                                   float *const *grad_loc_maps_h, float *const *grad_conf_maps_h, fdt_stream_t stream);
+int fdt_multibox_loss_forward_heads(const float *const *loc_maps_h, const float *const *conf_maps_h, const int *f_h, const int *f_w,
+                                    const int *neg_max_h, int n_levels, const float *priors, const float *gt, const int64_t *gt_off,
+                                    int64_t total_gt, int B, float threshold, int negpos_ratio, int bipartite, float var0, float var1,
+                                    float *losses, float *norm, float *loc_t, int64_t *conf_t, uint8_t *sel, float *loss_c_all,
+                                    void *ws, size_t ws_bytes, fdt_stream_t stream);
+int fdt_multibox_loss_backward_heads_dev(const float *const *loc_maps_h, const float *const *conf_maps_h, const int *f_h,
+                                         const int *f_w, const int *neg_max_h, int n_levels, const float *loc_t,
+                                         const int64_t *conf_t, const uint8_t *sel, const float *norm, const float *g_l_dev,
+                                         const float *g_c_dev, int B, float *const *grad_loc_maps_h,
+                                         float *const *grad_conf_maps_h, fdt_stream_t stream);
+
 /* ---- T2  IoU tracker association  (iouTracke_cal.py:126-155 loop, :174-176 flush) ----------------
  * dets[total,5] float64 rows [x1,y1,x2,y2,score]; frame_off[F+1] int64 (device); frames are 1-based in
  * the output.  Outputs (device): n_tracks[1] int64; track_off[total+1] int64 CSR offsets into
