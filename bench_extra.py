@@ -11,6 +11,7 @@
     python bench_extra.py torchref   # BASELINE.md 5.4: the reference's python-loop Detect restated in torch, on CUDA tensors and on the CPU
     python bench_extra.py heads      # SURVEY 8f rank 1: Detect straight from the per-level NCHW head maps, B=64 @640^2
     python bench_extra.py heads_train # SURVEY 8f rank 1: MultiBoxLoss (+ backward) straight from the head maps, B=32 @640^2 (config 3)
+    python bench_extra.py match_mine # fdt_match_encode and fdt_hard_negative_mine on their own (box_utils.match_*, DataEncoder.encode)
 
 Each prints one JSON line with device time (CUDA events, L2 flushed between repetitions), the algorithmic bytes of
 SURVEY 8(d) and the CPU oracle port timed on the host beside it."""
@@ -496,6 +497,80 @@ def heads_train():
                       "fused_fwd_algorithmic_bytes": B * 56 * N + 20 * G, "fused_bwd_algorithmic_bytes": B * 89 * N,
                       "fused_bwd_ms": ms_bwd, "fused_bwd_gbs": B * 89 * N / (ms_bwd * 1e-3) / 1e9,
                       "materialisation_removed_bytes": {"forward": B * 56 * N, "backward": B * 72 * N}}))
+
+
+def match_mine():
+    """The standalone entries, which share the fused forward's kernels: fdt_match_encode at config 3 (B=32, N=34,125, both matchers)
+    and as FaceBoxes' DataEncoder.encode calls it (B=1, the 21,824 default boxes, 10 GT boxes, bipartite); fdt_hard_negative_mine
+    (B=32, N=34,125) on the fused forward's loss_c of config 3 and on rows of ties, equal zeros and quarter steps.  outputs_sha1
+    identifies the outputs, so that two builds can be compared."""
+    import hashlib
+    from fdt_b200.layers.modules.multibox_loss import pack_targets
+    L = _lib.lib(); st = _lib.stream_ptr()
+    dev = torch.device("cuda")
+
+    def sha(*ts):
+        h = hashlib.sha1()
+        for t in ts:
+            h.update(t.cpu().numpy().tobytes())
+        return h.hexdigest()[:16]
+
+    def match_case(pri_np, gt, off, total, B, bip):
+        N = pri_np.shape[0]
+        p = torch.from_numpy(pri_np).to(dev)
+        lt = torch.empty((B, N, 4), device=dev); ct = torch.empty((B, N), dtype=torch.int64, device=dev)
+        bti = torch.empty((B, N), dtype=torch.int32, device=dev); bto = torch.empty((B, N), device=dev)
+        ws = _lib.workspace(L.fdt_match_workspace_bytes(B, N, total), dev, "mm")
+
+        def run():
+            _lib.check(L.fdt_match_encode(p.data_ptr(), gt.data_ptr(), off.data_ptr(), total, B, N, 0.35, 0.1, 0.2, bip, lt.data_ptr(),
+                                          ct.data_ptr(), bti.data_ptr(), bto.data_ptr(), ws.data_ptr(), ws.numel(), st))
+        run(); torch.cuda.synchronize()
+        ms, ms_min = timed(run)
+        return {"ms": ms, "ms_min": ms_min, "outputs_sha1": sha(lt, ct, bti, bto)}
+
+    res = {}
+    B = 32
+    pri = synth.priors_numpy(640, 640); N = pri.shape[0]
+    _, _, targets = synth.multibox_inputs(B, pri, 3030, 0, 200)
+    gt, off, G = pack_targets([torch.from_numpy(t).to(dev) for t in targets], dev)
+    for bip in (0, 1):
+        res[f"match_b32_config3_{'bipartite' if bip else 'default'}"] = match_case(pri, gt, off, G, B, bip)
+    fb = orc.facebox_default_boxes()
+    g10 = torch.from_numpy(synth.gt_boxes(10, np.random.Generator(np.random.PCG64(7)))).to(dev)
+    res["match_b1_faceboxes_bipartite"] = match_case(fb, g10, torch.tensor([0, 10], dtype=torch.int64, device=dev), 10, 1, 1)
+
+    # mining inputs: the loss_c and positives of the fused forward (config 3, default matcher), and the tie-heavy rows
+    loc, conf, _ = synth.multibox_inputs(B, pri, 3030, 0, 200)
+    l, c, p = (torch.from_numpy(a).to(dev) for a in (loc, conf, pri))
+    lca = torch.empty((B, N), device=dev); ct = torch.empty((B, N), dtype=torch.int64, device=dev)
+    ws = _lib.workspace(L.fdt_multibox_workspace_bytes(B, N, 2, G), dev, "mmf")
+    _lib.check(L.fdt_multibox_loss_forward(l.data_ptr(), c.data_ptr(), p.data_ptr(), gt.data_ptr(), off.data_ptr(), G, B, N, 2, 0.35, 3, 0,
+                                           0.1, 0.2, torch.empty(2, device=dev).data_ptr(), torch.empty(1, device=dev).data_ptr(),
+                                           torch.empty((B, N, 4), device=dev).data_ptr(), ct.data_ptr(),
+                                           torch.empty((B, N), dtype=torch.uint8, device=dev).data_ptr(), lca.data_ptr(), ws.data_ptr(),
+                                           ws.numel(), st))
+    rng = np.random.Generator(np.random.PCG64(34125 + 50))
+    lc_t = rng.uniform(0, 5, (B, N)).astype(np.float32)
+    lc_t[1::3] = np.round(lc_t[1::3] * 4) / 4
+    lc_t[2::3, ::2] = 0.0
+    pos_t = np.zeros((B, N), bool)
+    for b in range(B):
+        pos_t[b, rng.permutation(N)[:50]] = True
+    lc_t[pos_t] = 0
+    for name, lc, ps in (("mine_b32_config3_loss_c", lca, (ct > 0).to(torch.uint8)),
+                         ("mine_b32_ties", torch.from_numpy(lc_t).to(dev), torch.from_numpy(pos_t.astype(np.uint8)).to(dev))):
+        neg = torch.empty((B, N), dtype=torch.uint8, device=dev)
+        ws = _lib.workspace(L.fdt_mine_workspace_bytes(B, N), dev, "mm")
+
+        def run():
+            _lib.check(L.fdt_hard_negative_mine(lc.data_ptr(), ps.data_ptr(), B, N, 3, neg.data_ptr(), ws.data_ptr(), ws.numel(), st))
+        run(); torch.cuda.synchronize()
+        ms, ms_min = timed(run)
+        res[name] = {"ms": ms, "ms_min": ms_min, "outputs_sha1": sha(neg)}
+    print(json.dumps({"workload": "fdt_match_encode (B=32 config 3 default/bipartite; B=1 FaceBoxes 21,824 boxes, 10 GT, bipartite) and "
+                      "fdt_hard_negative_mine (B=32, N=34,125: config 3 loss_c; tie-heavy rows)", "device": torch.cuda.get_device_name(),
+                      "results": res}))
 
 
 if __name__ == "__main__":

@@ -26,16 +26,22 @@ def layers():
 
 def gpu_match(bip, thr, gt, pri, want_best=True):
     """fdt_match_encode for one image -> loc_t, conf_t, best_truth_idx, best_truth_overlap (numpy)."""
+    return tuple(a[0] for a in gpu_match_batch(bip, thr, [gt], pri))
+
+
+def gpu_match_batch(bip, thr, gts, pri):
+    """fdt_match_encode for len(gts) images in one call -> loc_t, conf_t, best_truth_idx, best_truth_overlap [B,N,...] (numpy)."""
     from fdt_b200 import _lib
     dev = torch.device("cuda", torch.cuda.current_device())
-    N = pri.shape[0]
-    g = cu(gt.astype(np.float32)); p = cu(pri)
-    off = torch.tensor([0, gt.shape[0]], dtype=torch.int64, device=dev)
-    lt = torch.empty((N, 4), dtype=torch.float32, device=dev); ct = torch.empty(N, dtype=torch.int64, device=dev)
-    bti = torch.empty(N, dtype=torch.int32, device=dev); bto = torch.empty(N, dtype=torch.float32, device=dev)
+    B, N = len(gts), pri.shape[0]
+    gt = np.concatenate(gts).astype(np.float32)
+    g = cu(gt); p = cu(pri)
+    off = torch.tensor(np.cumsum([0] + [t.shape[0] for t in gts]), dtype=torch.int64, device=dev)
+    lt = torch.empty((B, N, 4), dtype=torch.float32, device=dev); ct = torch.empty((B, N), dtype=torch.int64, device=dev)
+    bti = torch.empty((B, N), dtype=torch.int32, device=dev); bto = torch.empty((B, N), dtype=torch.float32, device=dev)
     L = _lib.lib()
-    ws = _lib.workspace(L.fdt_match_workspace_bytes(1, N, gt.shape[0]), dev, "t")
-    _lib.check(L.fdt_match_encode(p.data_ptr(), g.data_ptr(), off.data_ptr(), gt.shape[0], 1, N, thr, VAR[0], VAR[1], int(bip),
+    ws = _lib.workspace(L.fdt_match_workspace_bytes(B, N, gt.shape[0]), dev, "t")
+    _lib.check(L.fdt_match_encode(p.data_ptr(), g.data_ptr(), off.data_ptr(), gt.shape[0], B, N, thr, VAR[0], VAR[1], int(bip),
                                   lt.data_ptr(), ct.data_ptr(), bti.data_ptr(), bto.data_ptr(), ws.data_ptr(), ws.numel(),
                                   _lib.stream_ptr()))
     return npy(lt), npy(ct), npy(bti), npy(bto)
@@ -56,15 +62,21 @@ def test_match_golden(golden, tag, bip):
     np.testing.assert_allclose(lt, o_lt, rtol=1e-6, atol=1e-7)
 
 
-@pytest.mark.parametrize("G,bip,seed", [(1, 0, 1), (200, 0, 2), (200, 1, 3), (257, 1, 4), (700, 0, 5), (1968, 1, 6)])
+@pytest.mark.parametrize("G,bip,seed", [(1, 0, 1), (200, 0, 2), (200, 1, 3), (257, 1, 4), (700, 0, 5), (1968, 1, 6),
+                                        ((300, 0, 120), 0, 7), ((300, 0, 120), 1, 7)])
 def test_match_production_size_vs_oracle(G, bip, seed):
-    """N = 34,125; G up to the WIDER maximum (1,968 faces) -> several shared-memory GT tiles."""
+    """N = 34,125; G up to the WIDER maximum (1,968 faces) -> several shared-memory GT tiles.  A tuple of G: one call for that
+    many images (gt_off beyond the first image), one of them without GT boxes (all background, zeros everywhere)."""
     pri = synth.priors_numpy(640, 640)
-    gt = synth.gt_boxes(G, np.random.Generator(np.random.PCG64(seed)))
-    lt, ct, bti, bto = gpu_match(bip, 0.35, gt, pri)
-    o_lt, o_ct, o_bti, o_bto = orc.match(bip, 0.35, gt[:, :4], pri, VAR, gt[:, 4])
-    assert np.array_equal(ct, o_ct) and np.array_equal(bti, o_bti) and np.array_equal(bto, o_bto)
-    np.testing.assert_allclose(lt, o_lt, rtol=1e-6, atol=1e-7)
+    rng = np.random.Generator(np.random.PCG64(seed))
+    gts = [synth.gt_boxes(g, rng) for g in (G if isinstance(G, tuple) else (G,))]
+    for gt, (lt, ct, bti, bto) in zip(gts, zip(*gpu_match_batch(bip, 0.35, gts, pri))):
+        if gt.shape[0] == 0:
+            assert not lt.any() and not ct.any() and not bti.any() and not bto.any()
+            continue
+        o_lt, o_ct, o_bti, o_bto = orc.match(bip, 0.35, gt[:, :4], pri, VAR, gt[:, 4])
+        assert np.array_equal(ct, o_ct) and np.array_equal(bti, o_bti) and np.array_equal(bto, o_bto)
+        np.testing.assert_allclose(lt, o_lt, rtol=1e-6, atol=1e-7)
 
 
 def test_match_duplicate_gt_ties(golden):
@@ -115,10 +127,18 @@ def test_mining_on_reference_loss_bit_exact(golden, bip):
 @pytest.mark.parametrize("N,npos,ratio", [(34125, 50, 3), (34125, 0, 3), (34125, 20000, 3), (87360, 300, 3), (1000, 10, 7), (33, 4, 3)])
 def test_mining_vs_oracle_including_ties(N, npos, ratio):
     rng = np.random.Generator(np.random.PCG64(N + npos))
-    B = 3
+    B = 5
     lc = rng.uniform(0, 5, (B, N)).astype(np.float32)
     lc[1] = np.round(lc[1] * 4) / 4                         # heavy ties: boundary value duplicated
     lc[2, ::2] = 0.0
+    # the rest of the float range, which the mining histogram clamps into its first and last bins: NaN of either sign, negatives,
+    # values below 2^-8 down to subnormals, values above 2^8, infinities (no -0.0: the reference's sort ties it with +0.0)
+    nan2 = np.array([0x7FC00000, 0xFFC00000], np.uint32).view(np.float32)
+    kinds = np.stack([nan2[rng.integers(0, 2, N)], -rng.uniform(1e-6, 1e3, N),
+                      rng.uniform(0, 2.0 ** -8, N) * 10.0 ** -rng.integers(0, 40, N), rng.uniform(2.0 ** 8, 2.0 ** 30, N),
+                      np.where(rng.random(N) < 0.5, np.inf, -np.inf)]).astype(np.float32)
+    lc[3] = kinds[rng.integers(0, 5, N), np.arange(N)]
+    lc[4] = 1.5                                             # one value: every prior in the cutoff bin
     pos = np.zeros((B, N), bool)
     for b in range(B):
         pos[b, rng.permutation(N)[:npos]] = True
