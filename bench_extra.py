@@ -12,6 +12,8 @@
     python bench_extra.py heads      # SURVEY 8f rank 1: Detect straight from the per-level NCHW head maps, B=64 @640^2
     python bench_extra.py heads_train # SURVEY 8f rank 1: MultiBoxLoss (+ backward) straight from the head maps, B=32 @640^2 (config 3)
     python bench_extra.py match_mine # fdt_match_encode and fdt_hard_negative_mine on their own (box_utils.match_*, DataEncoder.encode)
+    python bench_extra.py track_stream # online tracker: V in {1, 64, 148} streams x 2,000 config-4 frames, one frame per stream per
+                                     # step, vs the offline tracker per video; Detect B=64 @640^2 + step_detections vs Detect alone
 
 Each prints one JSON line with device time (CUDA events, L2 flushed between repetitions), the algorithmic bytes of
 SURVEY 8(d) and the CPU oracle port timed on the host beside it."""
@@ -571,6 +573,145 @@ def match_mine():
     print(json.dumps({"workload": "fdt_match_encode (B=32 config 3 default/bipartite; B=1 FaceBoxes 21,824 boxes, 10 GT, bipartite) and "
                       "fdt_hard_negative_mine (B=32, N=34,125: config 3 loss_c; tie-heavy rows)", "device": torch.cuda.get_device_name(),
                       "results": res}))
+
+
+def card():
+    """name and power limit of the GPU the numbers of this run come from"""
+    import subprocess
+    try:
+        pl = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", str(torch.cuda.current_device())],
+                            capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception:
+        pl = "unknown"
+    return {"device": torch.cuda.get_device_name(), "power_limit": pl}
+
+
+def track_stream():
+    """Online multi-stream tracker (StreamTracker / fdt_track_stream_step): V in {1, 64, 148} streams x 2,000 config-4-shaped
+    frames each (one seed per stream), one frame per stream per step, steps back to back (eagerly through the C ABI, and replayed
+    from one CUDA graph holding all steps); against the same videos through the offline fdt_iou_track, one call per video, back to
+    back; and the live pipeline Detect (B=64 @640^2) + step_detections per step against Detect alone."""
+    from fdt_b200 import tracker as T
+    from fdt_b200.layers import Detect
+    L = _lib.lib()
+    dev = torch.device("cuda")
+    st_ptr = _lib.stream_ptr
+    F, MAXD = 2000, 300
+    res = {}
+    for V in (1, 64, 148):
+        videos = [synth.tracker_frames(F=F, seed=4040 + v, d_lo=1, d_hi=300, n_objects=300, empty_every=1000) for v in range(V)]
+        steps = []                                               # per step: packed rows of the V current frames (device)
+        for f in range(F):
+            d, o = T.pack_frames([videos[v][f] for v in range(V)])
+            steps.append((torch.from_numpy(d).to(dev), torch.from_numpy(o).to(dev)))
+        tr = T.StreamTracker(V, MAXD)
+        rt = torch.empty(max(int(s[0].shape[0]) for s in steps), dtype=torch.int64, device=dev)
+        rec = tr._records()
+
+        def step(s):
+            d, o = steps[s]
+            _lib.check(L.fdt_track_stream_step(tr._state.data_ptr(), V, MAXD, d.data_ptr(), o.data_ptr(), None, rt.data_ptr(),
+                                               rec["fin_count"].data_ptr(), rec["fin_index"].data_ptr(), rec["fin_track"].data_ptr(),
+                                               rec["fin_start"].data_ptr(), rec["fin_len"].data_ptr(), rec["fin_max"].data_ptr(),
+                                               tr._ws.data_ptr(), tr._ws.numel(), st_ptr()))
+
+        def reinit():
+            _lib.check(L.fdt_track_stream_init(tr._state.data_ptr(), tr._state.numel(), V, MAXD, 0, 0.4, 0.6, 5, st_ptr()))
+
+        def eager():
+            for s in range(F):
+                step(s)
+        reinit(); eager(); torch.cuda.synchronize()             # warm-up
+        t_eager = []
+        for _ in range(3):
+            reinit(); torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(); eager(); e1.record(); torch.cuda.synchronize()
+            t_eager.append(e0.elapsed_time(e1))
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.stream(side):
+            reinit()
+        torch.cuda.current_stream().wait_stream(side)
+        with torch.cuda.graph(g):
+            eager()
+        t_graph = []
+        for _ in range(3):
+            reinit(); torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(); g.replay(); e1.record(); torch.cuda.synchronize()
+            t_graph.append(e0.elapsed_time(e1))
+        del g
+
+        # parity: every stream's steps + flush against offline fdt_iou_track on its video (row grouping, start, length, max)
+        reinit()
+        ids, recs = [], []
+        for s in range(F):
+            o = tr.step(*steps[s]); ids.append(o["row_track"]); recs.append(o)
+        recs.append(tr.flush())
+        ids_h = [x.cpu().numpy() for x in ids]
+        recs_h = [{k: t.cpu().numpy() for k, t in r.items() if k != "row_track"} for r in recs]
+        offs_h = [s[1].cpu().numpy() for s in steps]
+        same = True
+        for v in range(V):
+            d, o = T.pack_frames(videos[v])
+            t_off, t_dets, t_start, t_max = (x.cpu().numpy() for x in T.iou_track_raw(d, o))
+            lab = np.full(int(o[-1]), -1, np.int64)
+            lab[t_dets] = np.repeat(np.arange(len(t_start)), np.diff(t_off))
+            idv = np.concatenate([ids_h[s][offs_h[s][v]:offs_h[s][v + 1]] for s in range(F)])
+            fin = [(int(r["fin_index"][v, k]), int(r["fin_track"][v, k]), int(r["fin_start"][v, k]), int(r["fin_len"][v, k]),
+                    float(r["fin_max"][v, k])) for r in recs_h for k in range(int(r["fin_count"][v]))]
+            fin.sort()
+            ok = [x[0] for x in fin] == list(range(len(t_start)))
+            ok = ok and all((x[2], x[3], x[4]) == (int(t_start[i]), int(t_off[i + 1] - t_off[i]), float(t_max[i])) for i, x in enumerate(fin))
+            idmap = np.full(int(idv.max(initial=0)) + 2, -1, np.int64)
+            idmap[[x[1] for x in fin]] = [x[0] for x in fin]
+            lab2 = idmap[idv]
+            same = same and ok and np.array_equal(lab, lab2)
+        status = tr.status()
+
+        # what users do today: the offline tracker, one call per video, back to back
+        packed = []
+        for v in range(V):
+            d, o = T.pack_frames(videos[v])
+            total = int(o[-1]); md = int(np.diff(o).max())
+            packed.append((torch.from_numpy(d).to(dev), torch.from_numpy(o).to(dev), total, md,
+                           torch.empty(max(int(L.fdt_iou_track_workspace_bytes(F, total, md)), 256), dtype=torch.uint8, device=dev)))
+        n = torch.zeros(1, dtype=torch.int64, device=dev)
+        tot_max = max(p[2] for p in packed)
+        t_off = torch.zeros(tot_max + 2, dtype=torch.int64, device=dev); t_dets = torch.zeros(tot_max, dtype=torch.int64, device=dev)
+        t_start = torch.zeros(tot_max + 1, dtype=torch.int64, device=dev); t_max = torch.zeros(tot_max + 1, dtype=torch.float64, device=dev)
+
+        def offline():
+            for d, o, total, md, ws in packed:
+                _lib.check(L.fdt_iou_track(d.data_ptr(), o.data_ptr(), F, total, md, 0.4, 0.6, 5, n.data_ptr(), t_off.data_ptr(),
+                                           t_dets.data_ptr(), t_start.data_ptr(), t_max.data_ptr(), ws.data_ptr(), ws.numel(), st_ptr()))
+        ms_off, ms_off_min = timed(offline, reps=3, warm=1)
+        ge = min(t_graph)
+        res[f"V{V}"] = {"streams": V, "frames_per_stream": F, "detections": int(sum(int(s[1][-1]) for s in steps)),
+                        "step_us_eager": min(t_eager) * 1e3 / F, "step_us_graph": ge * 1e3 / F,
+                        "frames_per_s_graph": V * F / (ge * 1e-3), "frames_per_s_eager": V * F / (min(t_eager) * 1e-3),
+                        "offline_ms_all_videos": ms_off, "offline_frames_per_s": V * F / (ms_off * 1e-3),
+                        "offline_us_per_frame": ms_off * 1e3 / (V * F), "identical_to_offline": bool(same), "status": status}
+        del steps, packed, ids, recs
+        torch.cuda.empty_cache()
+
+    # live pipeline: Detect at the headline configuration + one step_detections per step
+    B = 64
+    pri = synth.priors_numpy(640, 640)
+    loc, conf = synth.detect_inputs(B, pri, 4242, 0.05)
+    det = Detect(2, 0, 750, 0.05, 0.3)
+    a = [torch.from_numpy(x).cuda() for x in (loc, conf, pri)]
+    live = T.StreamTracker(B)
+    ms_det, _ = timed(lambda: det(*a))
+    ms_live, _ = timed(lambda: live.step_detections(det(*a), 640.0, 640.0))
+    out = live.step_detections(det(*a), 640.0, 640.0)
+    res["live_detect_b64_640"] = {"detect_ms": ms_det, "detect_plus_step_ms": ms_live, "step_ms_added": ms_live - ms_det,
+                                  "rows_per_step": int(out["frame_off"][-1]), "status": live.status()}
+    print(json.dumps({"workload": "online multi-stream IoU tracker: V streams x 2,000 config-4-shaped frames, one frame per stream "
+                      "per step; offline fdt_iou_track per video for comparison; Detect B=64 @640^2 + step_detections",
+                      **card(), "results": res}))
 
 
 if __name__ == "__main__":

@@ -87,7 +87,14 @@ SIGNATURES = {
     "fdt_iou_track_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "fdt_iou_track": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _d, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fdt_iou_track_metric": (_i, [_vp, _vp, _i64, _i64, _i64, _i, _d, _d, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_track_stream_state_bytes": (_sz, [_i64, _i64]),
+    "fdt_track_stream_workspace_bytes": (_sz, [_i64, _i64]),
+    "fdt_track_stream_init": (_i, [_vp, _sz, _i64, _i64, _i, _d, _d, _i64, _vp]),
+    "fdt_track_stream_step": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_track_stream_flush": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "fdt_track_stream_status": (_i, [_vp, _vp, _vp]),
 }
+TRACK_STATUS_OVERFLOW, TRACK_STATUS_MISMATCH = 4, 8
 
 _lib = None
 _lock = threading.Lock()

@@ -363,6 +363,38 @@ int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, int64_t F
                          int64_t *n_tracks, int64_t *track_off, int64_t *track_dets, int64_t *track_start, double *track_max,
                          void *ws, size_t ws_bytes, fdt_stream_t stream);
 
+/* ---- T2  online multi-stream tracker: each step advances V independent videos by one frame (iouTracke_cal.py:117-155
+ * inside the video loop), with every stream's active tracks kept on the device in a caller-owned `state` buffer (256-byte
+ * aligned).  No call synchronises with the host, so a Detect -> step chain can be captured in a CUDA graph.  For every stream,
+ * its steps followed by its flush give exactly fdt_iou_track_metric on that stream's frames.
+ *   cap = 32 * ceil(max_dets_per_frame / 32) (<= 800 detections per frame always fit).  Every call repeats V and
+ *   max_dets_per_frame; a call whose values differ from the state's sets FDT_STATUS_TRACK_MISMATCH and changes nothing.
+ *   Track ids are stream-local, in creation order from 0 (new tracks of a frame in detection order), below 2^31.
+ *   Finish records, [V, cap] each, entries [0, fin_count[v]) valid, in the reference's finishing order: fin_index = the
+ *   track's index in tracks_finished (the offline "track ID"), fin_track = its id, fin_start (1-based frame), fin_len, fin_max. */
+#define FDT_STATUS_TRACK_OVERFLOW 4u   /* a stream's frame had more than cap rows: that frame was skipped (state unchanged, ids -1) */
+#define FDT_STATUS_TRACK_MISMATCH 8u   /* a call's V / max_dets_per_frame differ from the state's (or it was never initialised) */
+size_t fdt_track_stream_state_bytes(int64_t V, int64_t max_dets_per_frame);
+size_t fdt_track_stream_workspace_bytes(int64_t V, int64_t max_dets_per_frame);      /* candidate rows of one step */
+/* metric / sigma as fdt_iou_track_metric; every stream starts a new video */
+int fdt_track_stream_init(void *state, size_t state_bytes, int64_t V, int64_t max_dets_per_frame,
+                          int metric, double sigma, double sigma_h, int64_t t_min, fdt_stream_t stream);
+/* One frame per stream: dets = packed float64 rows, frame_off[V+1] (device; what fdt_detections_to_frames_count/_pack write for a
+ * [V,C,top_k,5] Detect output).  advance[V] (NULL = all): 0 = the stream has no frame this call, its state is untouched -- not the
+ * same as an empty frame (D = 0: every active track is silently dropped).  row_track[frame_off[V]] = the id of the track each row
+ * joined or started (-1 for the rows of a stream that was not advanced or whose frame was over capacity). */
+int fdt_track_stream_step(void *state, int64_t V, int64_t max_dets_per_frame, const double *dets, const int64_t *frame_off,
+                          const uint8_t *advance, int64_t *row_track, int32_t *fin_count, int64_t *fin_index,
+                          int64_t *fin_track, int64_t *fin_start, int64_t *fin_len, double *fin_max,
+                          void *ws, size_t ws_bytes, fdt_stream_t stream);
+/* end of video (iouTracke_cal.py:174-176: len >= t_min) for the streams with streams[v] != 0 (NULL = all), the same records
+ * (fin_count[v] = 0 elsewhere); those slots then start a new video */
+int fdt_track_stream_flush(void *state, int64_t V, int64_t max_dets_per_frame, const uint8_t *streams, int32_t *fin_count,
+                           int64_t *fin_index, int64_t *fin_track, int64_t *fin_start, int64_t *fin_len, double *fin_max,
+                           fdt_stream_t stream);
+/* sticky FDT_STATUS_TRACK_* bits of the state (0 = fine); synchronises `stream`. */
+int fdt_track_stream_status(const void *state, fdt_stream_t stream, uint32_t *status_h);
+
 #ifdef __cplusplus
 }
 #endif
