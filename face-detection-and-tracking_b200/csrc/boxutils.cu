@@ -85,7 +85,7 @@ __global__ void k_pairwise(const T *__restrict__ a, int64_t A, const T *__restri
     }
 }
 
-// utils/calc_performance.py:34-51 calculate_distance (float64); `dis ** 0.25` is pow(dis, 0.25) like numpy
+// utils/calc_performance.py:34-51 calculate_distance (float64); `dis ** 0.25` correctly rounded, as the tracker computes it
 __global__ void k_pairwise_distance_f64(const double *__restrict__ a, int64_t A, const double *__restrict__ b, int64_t B, double *__restrict__ out)
 {
     int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -97,7 +97,7 @@ __global__ void k_pairwise_distance_f64(const double *__restrict__ a, int64_t A,
     const double dx = cbx - cax, dy = cby - cay;
     const double dz = ((adx - bdx) + (ady - bdy)) / 2;
     const double dis = __dadd_rn(__dadd_rn(__dmul_rn(dz, dz), __dmul_rn(dx, dx)), __dmul_rn(dy, dy));      // no FMA, numpy operand order
-    out[i * B + j] = pow(dis, 0.25);
+    out[i * B + j] = fdt_qroot_cr(dis);
 }
 
 // utils/calc_performance.py:77-92 calc_pr: one thread per prediction, max IoU over the truth boxes (given as x, y, w, h)

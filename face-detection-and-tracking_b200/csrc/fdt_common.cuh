@@ -48,6 +48,37 @@ constexpr int FDT_NUM_SMS = 148;            // B200
 constexpr int FDT_SMEM_MAX = 232448;        // 227 KB opt-in dynamic shared memory per CTA
 
 // ---- device helpers -------------------------------------------------------------------------
+// sign of (r + h)^4 - x, with (r + h)^2 and its square carried in double-double (error ~2^-100 relative; h = half an ulp of r)
+__device__ __forceinline__ int fdt_qroot_side(double r, double h, double x)
+{
+    const double p = __dmul_rn(r, r), pe = fma(r, r, -p);
+    const double b = __dmul_rn(2.0 * r, h), c = __dmul_rn(h, h);                     // exact: h is a power of two
+    const double s = __dadd_rn(p, b), bb = __dsub_rn(s, p);
+    const double e1 = __dadd_rn(__dsub_rn(p, __dsub_rn(s, bb)), __dsub_rn(b, bb));   // two-sum error of p + b
+    const double lo0 = __dadd_rn(__dadd_rn(pe, e1), c);
+    const double hi = __dadd_rn(s, lo0), lo = __dsub_rn(lo0, __dsub_rn(hi, s));
+    const double q = __dmul_rn(hi, hi), qe = fma(hi, hi, -q);
+    const double d = __dadd_rn(__dsub_rn(q, x), __dadd_rn(qe, __dmul_rn(2.0 * hi, lo)));
+    return (d > 0.0) - (d < 0.0);
+}
+// x ** 0.25 correctly rounded (utils/calc_performance.py:49 `dis ** 0.25`).  CUDA's pow is off by an ulp for about a quarter of all
+// inputs, exact fourth powers included (pow(k^4, 0.25) != k for 491 integers k < 8192), which moves ties and the `< sigma_dis`
+// edge of the tracker.  sqrt(sqrt(x)) is within one ulp; the neighbour across the nearer rounding midpoint is taken when
+// the midpoint's fourth power says so.  0, +inf, NaN and negative x give what pow gives.
+__device__ __forceinline__ double fdt_qroot_cr(double x)
+{
+    if (!(x > 0.0) || x == INFINITY) return sqrt(sqrt(x)) + 0.0;
+    double sc = 1.0;                                                                 // keep r^4 and its error terms in range
+    if (x < 0x1p-900) { x *= 0x1p800; sc = 0x1p-200; }
+    else if (x > 0x1p900) { x *= 0x1p-800; sc = 0x1p200; }
+    double r = sqrt(sqrt(x));
+    const long long rb = __double_as_longlong(r);                                   // r > 0 and normal here
+    const double up = __longlong_as_double(rb + 1), dn = __longlong_as_double(rb - 1);
+    if (fdt_qroot_side(r, 0.5 * (up - r), x) < 0) r = up;
+    else if (fdt_qroot_side(r, 0.5 * (dn - r), x) > 0) r = dn;
+    return r * sc;
+}
+
 // Order-preserving float -> uint32 map (larger float -> larger uint; +NaN above +inf like torch.sort).
 __device__ __forceinline__ uint32_t fdt_float_key(float f)
 {

@@ -29,8 +29,6 @@ namespace {
 
 constexpr int TR_THREADS = 1024;
 constexpr int OFF_CHUNK = 512;
-constexpr int TR_MAX_D = 1024;             // one thread per track / detection; shared memory caps this near 800
-                                           // (Detect emits at most top_k = 750 detections per frame)
 
 __device__ __forceinline__ double dmin_nan(double a, double b) { return (a != a || b != b) ? (double)NAN : (a < b ? a : b); }
 __device__ __forceinline__ double dmax_nan(double a, double b) { return (a != a || b != b) ? (double)NAN : (a > b ? a : b); }
@@ -49,15 +47,16 @@ __device__ __forceinline__ double iou_f64(const double *a, const double *b)
 }
 
 // utils/calc_performance.py:34-51 calculate_distance(box_a = detection, box_b = the track's last box): numpy operand order, no FMA,
-// `dis ** 0.25` = pow (within 2 ulp of numpy's: the association only differs if two candidates' distances agree to ~1e-15)
-__device__ __forceinline__ double distance_f64(const double *a, const double *b)
+// `dis ** 0.25` correctly rounded (fdt_qroot_cr), so ties and `< sigma_dis` at equality are decided like the reference.  Not inlined:
+// inlined into track_frame's re-rank and sequential path it made k_track_resolve and k_track_step spill.
+__device__ __noinline__ double distance_f64(const double *a, const double *b)
 {
     const double adx = a[2] - a[0], ady = a[3] - a[1], bdx = b[2] - b[0], bdy = b[3] - b[1];
     const double cax = (a[2] + a[0]) / 2, cay = (a[3] + a[1]) / 2, cbx = (b[2] + b[0]) / 2, cby = (b[3] + b[1]) / 2;
     const double dx = cbx - cax, dy = cby - cay;
     const double dz = ((adx - bdx) + (ady - bdy)) / 2;
     const double dis = __dadd_rn(__dadd_rn(__dmul_rn(dz, dz), __dmul_rn(dx, dx)), __dmul_rn(dy, dy));
-    return pow(dis, 0.25);
+    return fdt_qroot_cr(dis);
 }
 // association value, larger = better: the IoU (iouTracke_cal.py:131-134, matched iff > sigma_iou) or minus the distance
 // (:135-138: argmin, matched iff < sigma_dis  <=>  -distance > -sigma_dis).  First index on ties and first NaN wins either way.
@@ -77,6 +76,27 @@ __global__ void k_track_frame_of(const int64_t *__restrict__ frame_off, int64_t 
 // argmax order; 0xffff = none), [W+3] number of candidates.  The ranking is done here, for all frame pairs in parallel, so the
 // serial resolve kernel normally never evaluates an IoU.
 constexpr int ROW_EXTRA = 4;
+
+// dynamic shared memory of k_track_resolve (and of k_track_step: prefetch = 0) for cap = 32 * W rows per frame
+constexpr size_t resolve_smem(int W, int prefetch)
+{
+    const size_t cap = (size_t)W * 32;
+    size_t s = ((prefetch ? 2 : 1) * cap * (W + ROW_EXTRA) * 4 + 15) / 16 * 16;
+    s += sizeof(double) * ((prefetch ? 3 : 2) * cap * 5 + 2 * cap);
+    s += sizeof(int32_t) * 10 * cap;
+    return s;
+}
+constexpr size_t TR_SMEM_LIMIT = (size_t)FDT_SMEM_MAX - 1024;
+constexpr int tr_max_w()
+{
+    int W = 1;
+    while (resolve_smem(W + 1, 0) <= TR_SMEM_LIMIT) ++W;
+    return W;
+}
+// The one limit on rows per frame, offline and online: the largest cap whose frame state fits in shared memory (W = 27:
+// 224,640 B).  Frames of up to 608 rows (W = 19) also fit the prefetch layout.
+constexpr int TR_MAX_D = 32 * tr_max_w();
+static_assert(TR_MAX_D == 864 && TR_MAX_D <= TR_THREADS, "one thread per track / detection");
 
 // Where row g of k_track_mask takes its track box and its candidate frame from: row() returns false for a warp without a row,
 // otherwise it loads tb (the track's last box) and sets n0, D (the candidate rows dets[n0 .. n0 + D)); it may replace the rule.
@@ -556,14 +576,6 @@ TrackWs plan_track_ws(void *ws, int64_t total, int W)
     return t;
 }
 
-size_t resolve_smem(int W, int prefetch)
-{
-    const size_t cap = (size_t)W * 32;
-    size_t s = ((prefetch ? 2 : 1) * cap * (W + ROW_EXTRA) * 4 + 15) / 16 * 16;
-    s += sizeof(double) * ((prefetch ? 3 : 2) * cap * 5 + 2 * cap);
-    s += sizeof(int32_t) * 10 * cap;
-    return s;
-}
 
 // ---- online, multi-stream tracking: one frame per stream and call, the state carried between calls in a caller-owned buffer.
 // State = StreamHeader (256 bytes) + V slots.  A slot holds what k_track_resolve carries from frame f to frame f+1: the previous
@@ -759,12 +771,8 @@ int stream_check(const char *fn, const void *state, int64_t V, int64_t max_dets_
     FDT_REQUIRE(V >= 1 && max_dets_per_frame >= 0, FDT_E_INVALID, "%s: V=%lld, max_dets_per_frame=%lld", fn, (long long)V,
                 (long long)max_dets_per_frame);
     FDT_REQUIRE(V <= INT_MAX, FDT_E_UNSUPPORTED, "%s: V=%lld exceeds 2^31-1 streams", fn, (long long)V);
-    FDT_REQUIRE(max_dets_per_frame <= TR_MAX_D, FDT_E_UNSUPPORTED, "%s: %lld detections in one frame exceeds the limit of %d", fn,
-                (long long)max_dets_per_frame, TR_MAX_D);
-    const size_t smem = resolve_smem(stream_cap(max_dets_per_frame) / 32, 0);
-    FDT_REQUIRE(smem <= (size_t)FDT_SMEM_MAX - 1024, FDT_E_UNSUPPORTED,
-                "%s: %lld detections in one frame need %zu bytes of shared memory (limit %d; 800 per frame always fits)", fn,
-                (long long)max_dets_per_frame, smem, FDT_SMEM_MAX - 1024);
+    FDT_REQUIRE(max_dets_per_frame <= TR_MAX_D, FDT_E_UNSUPPORTED,
+                "%s: %lld detections in one frame exceed the limit of %d (shared memory)", fn, (long long)max_dets_per_frame, TR_MAX_D);
     return FDT_OK;
 }
 
@@ -773,6 +781,7 @@ int stream_check(const char *fn, const void *state, int64_t V, int64_t max_dets_
 FDT_API size_t fdt_iou_track_workspace_bytes(int64_t F, int64_t total, int64_t max_dets_per_frame)
 {
     (void)F;
+    if (total < 0 || max_dets_per_frame < 0 || max_dets_per_frame > TR_MAX_D) return 0;     // what fdt_iou_track_metric refuses
     int W = (int)((max_dets_per_frame + 31) / 32);
     if (W < 1) W = 1;
     return plan_track_ws(nullptr, total, W).bytes;
@@ -799,7 +808,8 @@ FDT_API int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, i
     FDT_REQUIRE(n_tracks && track_off, FDT_E_INVALID, "fdt_iou_track: null output pointer");
     FDT_REQUIRE(total < (1ll << 31), FDT_E_UNSUPPORTED, "fdt_iou_track: total=%lld exceeds 2^31-1", (long long)total);
     FDT_REQUIRE(max_dets_per_frame <= TR_MAX_D, FDT_E_UNSUPPORTED,
-                "fdt_iou_track: %lld detections in one frame exceeds the limit of %d", (long long)max_dets_per_frame, TR_MAX_D);
+                "fdt_iou_track: %lld detections in one frame exceed the limit of %d (shared memory)", (long long)max_dets_per_frame,
+                TR_MAX_D);
     if (F == 0 || total == 0) {
         FDT_CUDA(cudaMemsetAsync(n_tracks, 0, sizeof(int64_t), st));
         FDT_CUDA(cudaMemsetAsync(track_off, 0, sizeof(int64_t), st));
@@ -811,6 +821,8 @@ FDT_API int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, i
     if (W < 1) W = 1;
     TrackWs t = plan_track_ws(ws, total, W);
     FDT_REQUIRE(ws_bytes >= t.bytes, FDT_E_WORKSPACE, "fdt_iou_track: workspace %zu < %zu bytes", ws_bytes, t.bytes);
+    const int prefetch = resolve_smem(W, 1) <= TR_SMEM_LIMIT;
+    const size_t smem = resolve_smem(W, prefetch);       // <= TR_SMEM_LIMIT: W <= TR_MAX_D / 32 (checked above, before any CUDA call)
 
     FDT_CUDA(cudaMemsetAsync(t.fin_id, 0xff, (size_t)total * 4, st));
     k_track_frame_of<<<(unsigned)F, 128, 0, st>>>(frame_off, F, t.frame_of);
@@ -825,13 +837,9 @@ FDT_API int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, i
     P.n_tracks = n_tracks; P.track_off = track_off; P.track_start = track_start; P.track_max = track_max;
     const char *env = getenv("FDT_TRACK_FORCE_SLOW");
     P.force_slow = (env && env[0] == '1') ? 1 : 0;
-    P.prefetch = resolve_smem(W, 1) <= (size_t)FDT_SMEM_MAX - 1024;
-    const size_t smem = resolve_smem(W, P.prefetch);
-    FDT_REQUIRE(smem <= (size_t)FDT_SMEM_MAX - 1024, FDT_E_UNSUPPORTED,
-                "fdt_iou_track: %lld detections in one frame need %zu bytes of shared memory (limit %d; 800 per frame always fits)",
-                (long long)max_dets_per_frame, smem, FDT_SMEM_MAX - 1024);
+    P.prefetch = prefetch;
     FDT_CUDA(cudaFuncSetAttribute(k_track_resolve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_track_resolve<<<1, P.cap, smem, st>>>(P);      // cap = multiple of 32 >= max detections per frame, <= 1024
+    k_track_resolve<<<1, P.cap, smem, st>>>(P);      // cap = multiple of 32 >= max detections per frame, <= TR_MAX_D
     FDT_LAUNCH_CHECK();
     k_track_scatter<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(t.det_head, t.det_pos, t.fin_id, track_off, total, track_dets);
     FDT_LAUNCH_CHECK();

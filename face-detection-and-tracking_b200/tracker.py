@@ -107,10 +107,11 @@ class StreamTracker:
 
     A step returns device tensors: `row_track[rows]` int64, the stream-local id of the track each input row joined or started
     (ids count from 0 per video in creation order; -1 for the rows of a stream that was not advanced or whose frame had more than
-    max_dets_per_frame rows, which is then skipped and flagged -- see check()), and the tracks the step finished,
+    cap = 32 * ceil(max_dets_per_frame / 32) rows, which is then skipped and flagged -- see check(); frames of up to cap rows are
+    tracked), and the tracks the step finished,
     `fin_count[V]` int32 and `[V, cap]` records `fin_index` (index in the reference's tracks_finished = its "track ID"),
     `fin_track` (id), `fin_start` (1-based frame), `fin_len`, `fin_max`.  For every stream, steps + flush give exactly
-    iou_track(that stream's frames)."""
+    iou_track(that stream's frames).  max_dets_per_frame is at most 864."""
 
     def __init__(self, num_streams, max_dets_per_frame=800, sigma_iou=sigma_iou, sigma_h=sigma_h, t_min=t_min, use_iou=use_iou,
                  sigma_dis=sigma_dis, keep_history=False, device=None):
@@ -207,10 +208,10 @@ class StreamTracker:
         return bits.value
 
     def check(self):
-        """Raise if a frame was skipped for having more than max_dets_per_frame rows, or a call did not match the state."""
+        """Raise if a frame was skipped for having more than cap rows, or a call did not match the state."""
         bits = self.status()
         if bits & _lib.TRACK_STATUS_OVERFLOW:
-            raise RuntimeError(f"StreamTracker: a frame had more than max_dets_per_frame={self.max_d} rows and was skipped")
+            raise RuntimeError(f"StreamTracker: a frame had more than cap={self.cap} rows (max_dets_per_frame={self.max_d}) and was skipped")
         if bits & _lib.TRACK_STATUS_MISMATCH:
             raise RuntimeError("StreamTracker: a call's stream count or max_dets_per_frame did not match the state")
 

@@ -78,7 +78,7 @@ int fdt_calculate_iou(const float *box_a, int64_t A, const float *box_b, int64_t
 int fdt_calculate_iou_f64(const double *box_a, int64_t A, const double *box_b, int64_t B, double *out, fdt_stream_t stream);
 
 /* ---- (SURVEY 8f, Detect consumers)  utils.calc_performance.intersect / calculate_distance / calc_pr, float64 -----------------
- * (utils/calc_performance.py:4-31, 34-51, 77-92).  calculate_distance ends in pow(x, 0.25): compared at 1e-14 relative.
+ * (utils/calc_performance.py:4-31, 34-51, 77-92).  calculate_distance ends in x ** 0.25, correctly rounded.
  * calc_pr: predict[P, predict_stride >= 4] rows [x1,y1,x2,y2,(score..)], truth[T,4] rows [x,y,w,h] -> tf[P] int32 =
  * (max_t IoU > iou_thresh); NaN IoU makes the max NaN and the comparison false, as numpy does. */
 int fdt_intersect_f64(const double *box_a, int64_t A, const double *box_b, int64_t B, double *out, fdt_stream_t stream);
@@ -348,7 +348,10 @@ int fdt_multibox_loss_backward_heads_dev(const float *const *loc_maps_h, const f
  * dets[total,5] float64 rows [x1,y1,x2,y2,score]; frame_off[F+1] int64 (device); frames are 1-based in
  * the output.  Outputs (device): n_tracks[1] int64; track_off[total+1] int64 CSR offsets into
  * track_dets[total] int64 (global det rows in append order); track_start[total] int64;
- * track_max[total] float64 -- entries [0, n_tracks) are valid, in the reference's finishing order. */
+ * track_max[total] float64 -- entries [0, n_tracks) are valid, in the reference's finishing order.
+ * max_dets_per_frame must be at least every frame's row count; at most 864 rows per frame (the frame state of
+ * cap = 32 * ceil(max_dets_per_frame / 32) rows lives in shared memory), more return FDT_E_UNSUPPORTED before any CUDA call and
+ * fdt_iou_track_workspace_bytes returns 0 for them. */
 #define FDT_TRACK_IOU       0   /* use_iou = True:  calculate_iou, argmax, matched iff > sigma_iou   (iouTracke_cal.py:131-134) */
 #define FDT_TRACK_DISTANCE  1   /* use_iou = False: calculate_distance, argmin, matched iff < sigma_dis (iouTracke_cal.py:135-138) */
 size_t fdt_iou_track_workspace_bytes(int64_t F, int64_t total, int64_t max_dets_per_frame);
@@ -357,7 +360,7 @@ int fdt_iou_track(const double *dets, const int64_t *frame_off, int64_t F, int64
                   int64_t *n_tracks, int64_t *track_off, int64_t *track_dets, int64_t *track_start, double *track_max,
                   void *ws, size_t ws_bytes, fdt_stream_t stream);
 /* the same with the association rule of the reference's `use_iou` switch: metric FDT_TRACK_IOU (sigma = sigma_iou) or
- * FDT_TRACK_DISTANCE (sigma = sigma_dis; utils/calc_performance.py:34-51, `** 0.25` evaluated with pow, within 2 ulp of numpy). */
+ * FDT_TRACK_DISTANCE (sigma = sigma_dis; utils/calc_performance.py:34-51, `** 0.25` correctly rounded). */
 int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, int64_t F, int64_t total, int64_t max_dets_per_frame,
                          int metric, double sigma, double sigma_h, int64_t t_min,
                          int64_t *n_tracks, int64_t *track_off, int64_t *track_dets, int64_t *track_start, double *track_max,
@@ -367,7 +370,8 @@ int fdt_iou_track_metric(const double *dets, const int64_t *frame_off, int64_t F
  * inside the video loop), with every stream's active tracks kept on the device in a caller-owned `state` buffer (256-byte
  * aligned).  No call synchronises with the host, so a Detect -> step chain can be captured in a CUDA graph.  For every stream,
  * its steps followed by its flush give exactly fdt_iou_track_metric on that stream's frames.
- *   cap = 32 * ceil(max_dets_per_frame / 32) (<= 800 detections per frame always fit).  Every call repeats V and
+ *   cap = 32 * ceil(max_dets_per_frame / 32) (max_dets_per_frame <= 864, as offline; the size queries
+ *   return 0 above it).  Every call repeats V and
  *   max_dets_per_frame; a call whose values differ from the state's sets FDT_STATUS_TRACK_MISMATCH and changes nothing.
  *   Track ids are stream-local, in creation order from 0 (new tracks of a frame in detection order), below 2^31.
  *   Finish records, [V, cap] each, entries [0, fin_count[v]) valid, in the reference's finishing order: fin_index = the
