@@ -901,12 +901,18 @@ k_sort_nms(const SortNmsParams P)
     int k = min(n_c, P.nms_top_k);                           // box_utils.py:299 idx[-top_k:]   (FUSED: known after the first row scan)
     const bool prof = P.prof != nullptr && (blockIdx.x == 0 || P.prof_all) && tid == 0;
     const bool writer = crank == 0;                              // only one CTA of a cluster writes the results
-    long long pt = prof ? clock64() : 0, pacc[7] = {0, 0, 0, 0, 0, 0, 0};
-    const long long cta_t0 = (P.prof && tid == 0) ? clock64() : 0;
-    unsigned long long gt0 = 0;
-    if (P.prof && tid == 0) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt0));
-#define K3_STAMP(slot) do { if (P.prof) __syncthreads(); if (prof) { long long now_ = fdt_clock_after(s_warp); atomicAdd((unsigned long long *)&P.prof[slot], (unsigned long long)(now_ - pt)); pt = now_; } } while (0)
-#define K3_ACC(slot) do { if (P.prof) __syncthreads(); if (prof) { long long now_ = fdt_clock_after(s_warp); pacc[slot] += now_ - pt; pt = now_; } } while (0)
+    // Profiling state of thread 0 lives in shared memory: held in registers across the whole kernel, its clocks and per-phase
+    // accumulators made ptxas spill under the 64-register cap in every build, profiled or not.
+    __shared__ long long s_prof[10];                         // [0] last stamp, [1] CTA start clock, [2] CTA start globaltimer, [3 + q] phase q
+    long long *const pacc = s_prof + 3;
+    if (P.prof && tid == 0) {
+        unsigned long long g;
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
+        s_prof[0] = s_prof[1] = clock64(); s_prof[2] = (long long)g;
+        for (int q = 0; q < 7; ++q) pacc[q] = 0;
+    }
+#define K3_STAMP(slot) do { if (P.prof) __syncthreads(); if (prof) { long long now_ = fdt_clock_after(s_warp); atomicAdd((unsigned long long *)&P.prof[slot], (unsigned long long)(now_ - s_prof[0])); s_prof[0] = now_; } } while (0)
+#define K3_ACC(slot) do { if (P.prof) __syncthreads(); if (prof) { long long now_ = fdt_clock_after(s_warp); pacc[slot] += now_ - s_prof[0]; s_prof[0] = now_; } } while (0)
 
     // =========================================================== stage 1: top-k selection by bucket (counting) sort
     // Monotone score -> bucket map; counting sort by bucket, descending; only buckets that can reach rank < k are
@@ -947,47 +953,73 @@ k_sort_nms(const SortNmsParams P)
             if (FUSED) {
                 if (!scanned) {
                     scanned = true;
-                    // ballot compaction into the warp's queue; positions beyond the queue collapse onto its last entry and the
-                    // warp then visits ALL its priors in place on every pass: no bookkeeping inside the loop.  The U loads are issued
-                    // in NG groups, group g + 1 before group g is compacted: two groups in flight hide the HBM latency without the
-                    // register spills of all U at once.
+                    // Compaction into the warp's queue, one group of UG priors at a time: each thread counts its candidates, one warp
+                    // scan gives every thread its first queue position, and its candidates go to consecutive entries (thread-major
+                    // order inside a group; keys are unique, so the order inside the queue is free).  A group that would take the
+                    // queue past WQ_CAP is not stored: the warp then visits ALL its priors in place on every pass.  The U loads are
+                    // issued in NG groups, group g + 1 before group g is compacted: two groups in flight hide the HBM latency
+                    // without the register spills of all U at once.
                     constexpr int NG = FUSED ? 4 : 3, UG = U / NG;
                     const float qnan = __int_as_float(0x7fc00000);                          // never a candidate
-                    const unsigned lt = (1u << lane) - 1u;
                     const uint32_t qaddr = (uint32_t)__cvta_generic_to_shared(wq);
                     int run = 0;
                     float sv[NG][UG];
                     auto load_group = [&](const int g) {
                         const int i0 = tid + g * UG * K3_THREADS;
+                        const bool whole = (g + 1) * UG * K3_THREADS <= Nn;                  // (uniform) no prior of the group is past the row
                         if (Cc == 2) {                                                       // (addresses fold into the load immediates)
                             const float *p0 = crow + 2 * i0;
+                            if (whole) {
 #pragma unroll
-                            for (int u = 0; u < UG; ++u) sv[g][u] = i0 + u * K3_THREADS < Nn ? __ldg(p0 + 2 * u * K3_THREADS) : qnan;
+                                for (int u = 0; u < UG; ++u) sv[g][u] = __ldg(p0 + 2 * u * K3_THREADS);
+                            } else {
+#pragma unroll
+                                for (int u = 0; u < UG; ++u) sv[g][u] = i0 + u * K3_THREADS < Nn ? __ldg(p0 + 2 * u * K3_THREADS) : qnan;
+                            }
                         } else {
 #pragma unroll
                             for (int u = 0; u < UG; ++u) {
                                 const int i = i0 + u * K3_THREADS;
-                                sv[g][u] = i < Nn ? __ldg(crow + (int64_t)i * Cc) : qnan;
+                                sv[g][u] = (whole || i < Nn) ? __ldg(crow + (int64_t)i * Cc) : qnan;
                             }
                         }
                     };
-                    load_group(0);
+                    // POS: conf_thresh >= 0, so every candidate is a positive float and its key is its bits with the sign bit set
+                    auto compact = [&](auto pos_thr) {
+                        constexpr bool POS = decltype(pos_thr)::value;
+                        load_group(0);
 #pragma unroll
-                    for (int g = 0; g < NG; ++g) {
-                        if (g + 1 < NG) load_group(g + 1);
-                        const int i0 = tid + g * UG * K3_THREADS;
+                        for (int g = 0; g < NG; ++g) {
+                            if (g + 1 < NG) load_group(g + 1);
+                            // detection.py:64 strict gt; set.s32 gives -1 / 0, the count folds into 3-input adds and the stores
+                            // below re-test each score where it is stored (fewer predicate registers live than priors in a group)
+                            int cnt = 0;
 #pragma unroll
-                        for (int u = 0; u < UG; ++u) {
-                            const bool c = sv[g][u] > cthr;                                  // detection.py:64 strict gt
-                            const unsigned bal = __ballot_sync(0xffffffffu, c);
-                            const int idx = min(run + __popc(bal & lt), WQ_CAP - 1);
-                            // predicated store, no branch: a divergent `if` costs a BSSY / BRA / BSYNC triple per prior
-                            asm volatile("{ .reg .pred p; setp.ne.u32 p, %3, 0; @p st.shared.v2.u32 [%0], {%1, %2}; }"
-                                         :: "r"(qaddr + 8u * (uint32_t)idx), "r"((uint32_t)(i0 + u * K3_THREADS)), "r"(fdt_float_key(sv[g][u])),
-                                            "r"((unsigned)c) : "memory");
-                            run += __popc(bal);
+                            for (int u = 0; u < UG; ++u) {
+                                int m;
+                                asm("set.gt.s32.f32 %0, %1, %2;" : "=r"(m) : "f"(sv[g][u]), "f"(cthr));
+                                cnt -= m;
+                            }
+                            int inc = cnt;
+#pragma unroll
+                            for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
+                            const int tot = __shfl_sync(0xffffffffu, inc, 31);
+                            if (run + tot <= WQ_CAP) {                                          // (warp-uniform)
+                                uint32_t a = qaddr + 8u * (uint32_t)(run + inc - cnt);
+                                const uint32_t i0 = (uint32_t)(tid + g * UG * K3_THREADS);
+#pragma unroll
+                                for (int u = 0; u < UG; ++u) {
+                                    const uint32_t kk = POS ? (__float_as_uint(sv[g][u]) | 0x80000000u) : fdt_float_key(sv[g][u]);
+                                    // predicated store and advance, no branch: a divergent `if` costs a BSSY / BRA / BSYNC triple per prior
+                                    asm volatile("{ .reg .pred p; setp.gt.f32 p, %1, %2; @p st.shared.v2.u32 [%0], {%3, %4}; @p add.u32 %0, %0, 8; }"
+                                                 : "+r"(a) : "f"(sv[g][u]), "f"(cthr), "r"(i0 + u * K3_THREADS), "r"(kk) : "memory");
+                                }
+                            }
+                            run += tot;
                         }
-                    }
+                    };
+                    if (cthr >= 0.0f) compact(std::true_type{});
+                    else compact(std::false_type{});
                     wq_ovf = run > WQ_CAP;
                     wq_n = wq_ovf ? 0 : run;
                     __syncwarp();
@@ -1476,7 +1508,7 @@ k_sort_nms(const SortNmsParams P)
                     else if (!pend) { st = 1; status[id] = 1; }
                 }
                 if (!__syncthreads_or(st == 0)) break;       // one barrier per sweep; it also publishes the status bytes
-                if (prof && sweeps <= 4) { long long now_ = clock64(); P.prof[20 + sweeps] = now_ - pt; }
+                if (prof && sweeps <= 4) { long long now_ = clock64(); P.prof[20 + sweeps] = now_ - s_prof[0]; }
             }
         }
         K3_ACC(5);
@@ -1506,11 +1538,11 @@ k_sort_nms(const SortNmsParams P)
         atomicAdd((unsigned long long *)&P.prof[12], (unsigned long long)nkept); atomicAdd((unsigned long long *)&P.prof[13], (unsigned long long)k);
         atomicAdd((unsigned long long *)&P.prof[14], (unsigned long long)rounds); atomicAdd((unsigned long long *)&P.prof[15], (unsigned long long)sweeps);
         atomicAdd((unsigned long long *)&P.prof[30], 1ull);
-        atomicAdd((unsigned long long *)&P.prof[31], (unsigned long long)(clock64() - cta_t0));
+        atomicAdd((unsigned long long *)&P.prof[31], (unsigned long long)(clock64() - s_prof[1]));
     }
 
     // =========================================================== stage 3: outputs
-    if (P.prof && tid == 0 && blockIdx.x < 256) { unsigned long long gt1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt1)); atomicMin((unsigned long long *)&P.prof[40], gt0); atomicMax((unsigned long long *)&P.prof[41], gt0); atomicMin((unsigned long long *)&P.prof[42], gt1); atomicMax((unsigned long long *)&P.prof[43], gt1); P.prof[64 + blockIdx.x] = clock64() - cta_t0; P.prof[320 + blockIdx.x] = (long long)rounds * 100000 + k; }
+    if (P.prof && tid == 0 && blockIdx.x < 256) { unsigned long long gt1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt1)); atomicMin((unsigned long long *)&P.prof[40], (unsigned long long)s_prof[2]); atomicMax((unsigned long long *)&P.prof[41], (unsigned long long)s_prof[2]); atomicMin((unsigned long long *)&P.prof[42], gt1); atomicMax((unsigned long long *)&P.prof[43], gt1); P.prof[64 + blockIdx.x] = clock64() - s_prof[1]; P.prof[320 + blockIdx.x] = (long long)rounds * 100000 + k; }
     if (!writer) return;
     const bool gather = MODE == MODE_DETECT && P.peer_sig != nullptr;
     // Completion ticket (see the end of the kernel).  Fused call, local output, kept rows in shared memory: `done` only has to say
