@@ -575,6 +575,100 @@ def match_mine():
                       "results": res}))
 
 
+def heads_amp():
+    """Mixed-precision / channels_last head maps read in place vs today's conversion path (each map converted to fp32 NCHW first,
+    [m.float().contiguous() ...]), at the heads / heads_train shapes: Detect B=64 and MultiBoxLoss B=32 (config 3 ground truth),
+    both at 640x640 (N=34,125).  Cases: fp32 NCHW, bf16 NCHW and channels_last (converted and native), fp16 NCHW native.  Every
+    native result is checked equal to its conversion-path twin in the same run.  Bytes are algorithmic, from the shapes: Detect
+    reads the conf maps (4 channels x sizeof(T) per prior and image); the loss reads the loc and conf maps at sizeof(T) and writes
+    its targets as today (loc_t 16, conf_t 8, sel 1 bytes per prior and image)."""
+    from fdt_b200.layers import Detect, MultiBoxLoss
+    N = synth.priors_numpy(640, 640).shape[0]
+    pri = torch.from_numpy(synth.priors_numpy(640, 640)).cuda()
+
+    def make(B, seed, dtype, layout):
+        lm, cm, nm = synth.head_maps(B, 640, 640, seed)
+        out = []
+        for maps in (lm, cm):
+            ms = [torch.from_numpy(m).to(dtype).cuda() for m in maps]
+            out.append([m.contiguous(memory_format=torch.channels_last) for m in ms] if layout == "channels_last" else ms)
+        return out[0], out[1], nm
+
+    def convert(maps):
+        return [m.float().contiguous() for m in maps]
+    cases = [("fp32_nchw", torch.float32, "nchw", False), ("bf16_nchw_converted", torch.bfloat16, "nchw", True),
+             ("bf16_nchw_native", torch.bfloat16, "nchw", False), ("bf16_cl_converted", torch.bfloat16, "channels_last", True),
+             ("bf16_cl_native", torch.bfloat16, "channels_last", False), ("fp16_nchw_native", torch.float16, "nchw", False)]
+    res = {}
+    # ---- Detect, B = 64
+    B = 64
+    det = Detect(2, 0, 750, 0.05, 0.3)
+    ref = {}
+    for name, dtype, layout, conv in cases:
+        sets = [make(B, 6060 + i, dtype, layout) for i in range(2)]
+
+        def call(i):
+            lm, cm, nm = sets[i % 2]
+            return det.detect_heads(convert(lm) if conv else lm, convert(cm) if conv else cm, pri, nm)
+        key = (dtype, layout)
+        out = call(0)
+        if key in ref:
+            assert torch.equal(out, ref[key]), name
+        ref[key] = out
+        ms, ms_min = timed(lambda: call(0))
+        for i in range(8):
+            call(i)
+        torch.cuda.synchronize()
+        blocks = []
+        for _ in range(5):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda._sleep(2_000_000)
+            e0.record()
+            for i in range(50):
+                call(i)
+            e1.record()
+            torch.cuda.synchronize()
+            blocks.append(e0.elapsed_time(e1) / 50)
+        esz = torch.tensor([], dtype=dtype).element_size()
+        res["detect_b64_" + name] = {"isolated_ms": ms, "isolated_ms_min": ms_min, "back_to_back_ms": float(np.median(blocks)),
+                                     "conf_map_bytes": B * 4 * N * esz}
+    # ---- MultiBoxLoss, B = 32
+    B = 32
+    _, _, targets = synth.multibox_inputs(B, synth.priors_numpy(640, 640), 3030, 0, 200)
+    tg = [torch.from_numpy(t).cuda() for t in targets]
+    crit = MultiBoxLoss(2, 0.35, True, 0, True, 3, 0.35, False)
+    ref = {}
+    for name, dtype, layout, conv in cases:
+        lm0, cm0, nm = make(B, 3032, dtype, layout)
+        lm = [m.requires_grad_(True) for m in lm0]
+        cm = [m.requires_grad_(True) for m in cm0]
+
+        def fwd():
+            with torch.no_grad():
+                return crit.forward_heads(convert(lm) if conv else lm, convert(cm) if conv else cm, pri, tg, nm)
+
+        def fwd_bwd():
+            for m in lm + cm:
+                m.grad = None
+            ll, lc = crit.forward_heads(convert(lm) if conv else lm, convert(cm) if conv else cm, pri, tg, nm)
+            (ll + lc).backward()
+            return ll, lc
+        ll, lc = fwd_bwd()
+        got = (float(ll.detach()), float(lc.detach()), [m.grad.clone() for m in lm + cm])
+        key = (dtype, layout)
+        if key in ref:
+            assert got[:2] == ref[key][:2], name
+            assert all(torch.equal(a, b) for a, b in zip(got[2], ref[key][2])), name
+        ref[key] = got
+        ms_f, _ = timed(fwd)
+        ms_fb, _ = timed(fwd_bwd)
+        esz = torch.tensor([], dtype=dtype).element_size()
+        res["loss_b32_" + name] = {"forward_ms": ms_f, "forward_backward_ms": ms_fb,
+                                   "forward_bytes": B * N * (8 * esz + 16 + 8 + 1)}
+    print(json.dumps({"workload": "head maps as the network wrote them (bf16 / fp16, NCHW / channels_last) vs converted to fp32 NCHW; "
+                      "Detect B=64 and MultiBoxLoss B=32 @640x640", **card(), "results": res}))
+
+
 def card():
     """name and power limit of the GPU the numbers of this run come from"""
     import subprocess

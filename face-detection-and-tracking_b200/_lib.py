@@ -84,6 +84,12 @@ SIGNATURES = {
     "fdt_multibox_loss_forward_heads": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i64, _i, _f, _i, _i, _f, _f,
                                              _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fdt_multibox_loss_backward_heads_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "fdt_heads_to_loc_conf_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "fdt_detect_heads_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_heads_to_loc_conf_backward_ex": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "fdt_multibox_loss_forward_heads_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i64, _i, _f, _i, _i, _f, _f,
+                                                _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_multibox_loss_backward_heads_dev_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "fdt_iou_track_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "fdt_iou_track": (_i, [_vp, _vp, _i64, _i64, _i64, _d, _d, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fdt_iou_track_metric": (_i, [_vp, _vp, _i64, _i64, _i64, _i, _d, _d, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

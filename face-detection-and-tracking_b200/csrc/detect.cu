@@ -57,6 +57,7 @@ enum { MODE_DETECT = 0, MODE_NMS = 1 };
 
 // Materialises the reference's tensors: loc_out[B,N,4] and conf_out[B,N,2] (softmax applied iff `softmax`; the training
 // path keeps raw logits, pyramid.py:339-346).  Either output may be null.
+template <int F>
 __global__ void __launch_bounds__(256)
 k_heads_to_loc_conf(const HeadLevels h, const int N, const int softmax, float *__restrict__ loc_out, float *__restrict__ conf_out)
 {
@@ -64,11 +65,11 @@ k_heads_to_loc_conf(const HeadLevels h, const int N, const int softmax, float *_
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= N) return;
     if (conf_out) {
-        float2 x = head_logits(h, b, p);
+        float2 x = head_logits<F>(h, b, p);
         if (softmax) x = softmax2(x);
         reinterpret_cast<float2 *>(conf_out)[(int64_t)b * N + p] = x;
     }
-    if (loc_out) reinterpret_cast<float4 *>(loc_out)[(int64_t)b * N + p] = head_loc_row(h, b, p);
+    if (loc_out) reinterpret_cast<float4 *>(loc_out)[(int64_t)b * N + p] = head_loc_row<F>(h, b, p);
 }
 
 // ------------------------------------------------------------------------------------------- call sequencing
@@ -243,6 +244,7 @@ __device__ __forceinline__ unsigned detect_call_seq(const DetectSlots &S, unsign
 // 9 priors per thread: 15 tiles per 640x640 image, so that B = 64 is a single wave at 7 blocks per SM.
 constexpr int K2H_PER_THREAD = 9;
 constexpr int K2H_TILE = K2_THREADS * K2H_PER_THREAD;
+template <int F>
 __global__ void __launch_bounds__(K2_THREADS, 7)
 k_heads_threshold_compact(const HeadLevels hl, const int64_t N, const float thr, const float dcut,
                           const DetectSlots S, long long *prof)
@@ -272,7 +274,7 @@ k_heads_threshold_compact(const HeadLevels hl, const int64_t N, const float thr,
         const int64_t p = base + u * K2_THREADS + tid;
         bool maybe = false;
         if (p < N) {
-            const float2 lg = head_logits(hl, b, (int)p);
+            const float2 lg = head_logits<F>(hl, b, (int)p);
             maybe = (lg.y - lg.x) > dcut;
             s_x[u * K2_THREADS + tid] = ((unsigned long long)__float_as_uint(lg.y) << 32) | __float_as_uint(lg.x);
         }
@@ -780,7 +782,9 @@ __device__ __forceinline__ void csr_scan(int *a, int *s_warp)
 #else
 #define K3_BOUNDS __launch_bounds__(K3_THREADS, 1)
 #endif
-template <int MODE, int CL, bool FUSED>
+// HT = 1: MODE_DETECT with the loc rows gathered from head maps other than fp32 dense NCHW (HEAD_ANY, heads.cuh): in the
+// instantiations above their loads and widening would cost the 64-register kernel extra spill traffic
+template <int MODE, int CL, bool FUSED, int HT = 0>
 __global__ void K3_BOUNDS
 k_sort_nms(const SortNmsParams P)
 {
@@ -1259,7 +1263,8 @@ k_sort_nms(const SortNmsParams P)
                 key = skeys[j];
                 const uint32_t p = (uint32_t)key;
                 if (MODE == MODE_DETECT) {
-                    ld0 = P.loc ? __ldg(reinterpret_cast<const float4 *>(P.loc) + ((int64_t)b * P.N + p)) : head_loc_row(P.hl, b, (int)p);
+                    if constexpr (HT == 1) ld0 = head_loc_row<HEAD_ANY>(P.hl, b, (int)p);
+                    else ld0 = P.loc ? __ldg(reinterpret_cast<const float4 *>(P.loc) + ((int64_t)b * P.N + p)) : head_loc_row<HEAD_F32_NCHW>(P.hl, b, (int)p);
                     ld1 = __ldg(reinterpret_cast<const float4 *>(P.priors) + p);
                 } else {
                     ld0 = __ldg(reinterpret_cast<const float4 *>(P.boxes) + p);
@@ -1802,8 +1807,15 @@ int launch_sort_nms(SortNmsParams &P, int lists, int kcap, void *kept_ws, size_t
         ++na;
     }
     cfg.attrs = attr; cfg.numAttrs = na;
-    static FuncAttrCache cache_cl, cache_1, cache_f;
-    if (fused) {
+    static FuncAttrCache cache_cl, cache_1, cache_f, cache_cl_any, cache_1_any;
+    const bool head_any = MODE == MODE_DETECT && P.loc == nullptr && !P.hl.f32_nchw;
+    if (head_any && cluster) {
+        int rc = ensure_dyn_smem(k_sort_nms<MODE_DETECT, 2, false, 1>, cache_cl_any, sp.total); if (rc != FDT_OK) return rc;
+        FDT_CUDA(cudaLaunchKernelEx(&cfg, k_sort_nms<MODE_DETECT, 2, false, 1>, P));
+    } else if (head_any) {
+        int rc = ensure_dyn_smem(k_sort_nms<MODE_DETECT, 1, false, 1>, cache_1_any, sp.total); if (rc != FDT_OK) return rc;
+        FDT_CUDA(cudaLaunchKernelEx(&cfg, k_sort_nms<MODE_DETECT, 1, false, 1>, P));
+    } else if (fused) {
         int rc = ensure_dyn_smem(k_sort_nms<MODE_DETECT, 1, true>, cache_f, sp.total); if (rc != FDT_OK) return rc;
         FDT_CUDA(cudaLaunchKernelEx(&cfg, k_sort_nms<MODE_DETECT, 1, true>, P));
     } else if (cluster) {
@@ -1953,7 +1965,8 @@ static int threshold_compact_impl(const float *conf, const HeadLevels *heads, in
             float dcut = -INFINITY;
             if (conf_thresh > 1e-4f && conf_thresh < 1.0f - 1e-4f) dcut = logf(conf_thresh / (1.0f - conf_thresh)) - 1e-3f;
             else if (conf_thresh >= 1.0f - 1e-4f) dcut = 9.0f;          // sigmoid(9) < 1 - 1e-4: nothing at or below can pass
-            FDT_CUDA(cudaLaunchKernelEx(&cfg, k_heads_threshold_compact, hl, N_, conf_thresh, dcut, S, prof));
+            if (hl.f32_nchw) FDT_CUDA(cudaLaunchKernelEx(&cfg, k_heads_threshold_compact<HEAD_F32_NCHW>, hl, N_, conf_thresh, dcut, S, prof));
+            else             FDT_CUDA(cudaLaunchKernelEx(&cfg, k_heads_threshold_compact<HEAD_ANY>, hl, N_, conf_thresh, dcut, S, prof));
         }
         else if (C == 2) FDT_CUDA(cudaLaunchKernelEx(&cfg, k_threshold_compact<1>, conf, hl, N_, C, conf_thresh, S, prof));
         else             FDT_CUDA(cudaLaunchKernelEx(&cfg, k_threshold_compact<0>, conf, hl, N_, C, conf_thresh, S, prof));
@@ -2186,26 +2199,54 @@ FDT_API int fdt_detect(const float *loc, const float *conf, const float *priors,
 }
 
 // ---- head maps -> Detect (SURVEY 8f rank 1; pyramid.py:291-309, 331-338)
-FDT_API int fdt_heads_to_loc_conf(const float *const *loc_maps_h, const float *const *conf_maps_h,
-                                  const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, int B, int softmax,
-                                  float *loc_out, float *conf_out, fdt_stream_t stream)
+FDT_API int fdt_heads_to_loc_conf_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype,
+                                     const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, int B, int softmax,
+                                     float *loc_out, float *conf_out, fdt_stream_t stream)
 {
     HeadLevels hl;
     int64_t N = 0;
-    int rc = heads_fill(hl, "fdt_heads_to_loc_conf", loc_maps_h, conf_maps_h, f_h, f_w, neg_max_h, n_levels, &N);
+    int rc = heads_fill(hl, "fdt_heads_to_loc_conf", loc_maps_h, conf_maps_h, dtype, f_h, f_w, neg_max_h, n_levels, &N);
     if (rc != FDT_OK) return rc;
     FDT_REQUIRE(B >= 0, FDT_E_INVALID, "fdt_heads_to_loc_conf: B=%d", B);
     if (B == 0 || (!loc_out && !conf_out)) return FDT_OK;
     for (int l = 0; l < n_levels; ++l) {
-        FDT_REQUIRE(!loc_out || hl.loc[l], FDT_E_INVALID, "fdt_heads_to_loc_conf: loc map %d is null", l);
-        FDT_REQUIRE(!conf_out || hl.conf[l], FDT_E_INVALID, "fdt_heads_to_loc_conf: conf map %d is null", l);
+        FDT_REQUIRE(!loc_out || hl.loc[l].p, FDT_E_INVALID, "fdt_heads_to_loc_conf: loc map %d is null", l);
+        FDT_REQUIRE(!conf_out || hl.conf[l].p, FDT_E_INVALID, "fdt_heads_to_loc_conf: conf map %d is null", l);
     }
     FDT_REQUIRE((!loc_out || fdt_aligned(loc_out, 16)) && (!conf_out || fdt_aligned(conf_out, 8)), FDT_E_INVALID,
                 "fdt_heads_to_loc_conf: outputs need 16 / 8-byte alignment");
     dim3 g((unsigned)((N + 255) / 256), (unsigned)B);
-    k_heads_to_loc_conf<<<g, 256, 0, (cudaStream_t)stream>>>(hl, (int)N, softmax, loc_out, conf_out);
+    if (hl.f32_nchw) k_heads_to_loc_conf<HEAD_F32_NCHW><<<g, 256, 0, (cudaStream_t)stream>>>(hl, (int)N, softmax, loc_out, conf_out);
+    else             k_heads_to_loc_conf<HEAD_ANY><<<g, 256, 0, (cudaStream_t)stream>>>(hl, (int)N, softmax, loc_out, conf_out);
     FDT_LAUNCH_CHECK();
     return FDT_OK;
+}
+
+FDT_API int fdt_heads_to_loc_conf(const float *const *loc_maps_h, const float *const *conf_maps_h,
+                                  const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, int B, int softmax,
+                                  float *loc_out, float *conf_out, fdt_stream_t stream)
+{
+    fdt_head_map lm[FDT_MAX_LEVELS], cm[FDT_MAX_LEVELS];
+    return fdt_heads_to_loc_conf_ex(heads_nchw(lm, loc_maps_h, f_h, f_w, n_levels), heads_nchw(cm, conf_maps_h, f_h, f_w, n_levels),
+                                    FDT_DTYPE_F32, f_h, f_w, neg_max_h, n_levels, B, softmax, loc_out, conf_out, stream);
+}
+
+FDT_API int fdt_detect_heads_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype,
+                                const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, const float *priors,
+                                int B, int top_k, int nms_top_k, float conf_thresh, float nms_thresh, float var0, float var1,
+                                float *out, int32_t *counts, int64_t *kept_prior, void *ws, size_t ws_bytes, fdt_stream_t stream)
+{
+    HeadLevels hl;
+    int64_t N = 0;
+    int rc = heads_fill(hl, "fdt_detect_heads", loc_maps_h, conf_maps_h, dtype, f_h, f_w, neg_max_h, n_levels, &N);
+    if (rc != FDT_OK) return rc;
+    FDT_REQUIRE(loc_maps_h && conf_maps_h, FDT_E_INVALID, "fdt_detect_heads: null map arrays");
+    for (int l = 0; l < n_levels; ++l)
+        FDT_REQUIRE(hl.loc[l].p && hl.conf[l].p, FDT_E_INVALID, "fdt_detect_heads: map %d is null", l);
+    rc = threshold_compact_impl(nullptr, &hl, B, N, 2, conf_thresh, ws, ws_bytes, stream, out, counts, kept_prior, 0);
+    if (rc != FDT_OK) return rc;
+    return detect_sort_nms_impl(nullptr, &hl, priors, B, N, 2, top_k, nms_top_k, nms_thresh, var0, var1, out, counts, kept_prior,
+                                GatherArgs{}, ws, ws_bytes, stream);
 }
 
 FDT_API int fdt_detect_heads(const float *const *loc_maps_h, const float *const *conf_maps_h,
@@ -2213,17 +2254,10 @@ FDT_API int fdt_detect_heads(const float *const *loc_maps_h, const float *const 
                              int B, int top_k, int nms_top_k, float conf_thresh, float nms_thresh, float var0, float var1,
                              float *out, int32_t *counts, int64_t *kept_prior, void *ws, size_t ws_bytes, fdt_stream_t stream)
 {
-    HeadLevels hl;
-    int64_t N = 0;
-    int rc = heads_fill(hl, "fdt_detect_heads", loc_maps_h, conf_maps_h, f_h, f_w, neg_max_h, n_levels, &N);
-    if (rc != FDT_OK) return rc;
-    FDT_REQUIRE(loc_maps_h && conf_maps_h, FDT_E_INVALID, "fdt_detect_heads: null map arrays");
-    for (int l = 0; l < n_levels; ++l)
-        FDT_REQUIRE(hl.loc[l] && hl.conf[l], FDT_E_INVALID, "fdt_detect_heads: map %d is null", l);
-    rc = threshold_compact_impl(nullptr, &hl, B, N, 2, conf_thresh, ws, ws_bytes, stream, out, counts, kept_prior, 0);
-    if (rc != FDT_OK) return rc;
-    return detect_sort_nms_impl(nullptr, &hl, priors, B, N, 2, top_k, nms_top_k, nms_thresh, var0, var1, out, counts, kept_prior,
-                                GatherArgs{}, ws, ws_bytes, stream);
+    fdt_head_map lm[FDT_MAX_LEVELS], cm[FDT_MAX_LEVELS];
+    return fdt_detect_heads_ex(heads_nchw(lm, loc_maps_h, f_h, f_w, n_levels), heads_nchw(cm, conf_maps_h, f_h, f_w, n_levels),
+                               FDT_DTYPE_F32, f_h, f_w, neg_max_h, n_levels, priors, B, top_k, nms_top_k, conf_thresh, nms_thresh,
+                               var0, var1, out, counts, kept_prior, ws, ws_bytes, stream);
 }
 
 // Diagnostics: with FDT_K3_PROFILE=1 in the environment, CTA 0 of k_sort_nms records clock64 deltas per phase:

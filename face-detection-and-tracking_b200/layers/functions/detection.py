@@ -82,8 +82,8 @@ class Detect:
         pyramid.py:291-309, 331-332 are fused into the threshold kernel, and NMS gathers the loc rows it decodes
         from the maps -- loc[B,N,4] / conf[B,N,2] are never materialised.  Same output as
         self(*heads_to_loc_conf(loc_maps, conf_maps), prior_data)."""
-        from .heads import _level_args
-        dev, num, num_priors, keep, (lp, cp, fh, fw, nm, L) = _level_args(loc_maps, conf_maps, neg_max)
+        from .heads import _head_args
+        dev, num, num_priors, keep, (ld, cd, dt, fh, fw, nm, L) = _head_args(loc_maps, conf_maps, neg_max)
         if self.num_classes != 2:
             raise NotImplementedError("detect_heads: the max-in-out heads are two-class (background / face)")
         if prior_data.size(0) != num_priors:
@@ -95,10 +95,10 @@ class Detect:
             kept = torch.empty((num, 2, self.top_k), dtype=torch.int64, device=dev) if return_aux else None
             Lb = _lib.lib()
             ws = self._workspaces.get(num, num_priors, 2, dev)
-            _lib.check(Lb.fdt_detect_heads(lp, cp, fh, fw, nm, L, _lib.ptr(pri), num, int(self.top_k), int(self.nms_top_k),
-                                           float(self.conf_thresh), float(self.nms_thresh), float(self.variance[0]),
-                                           float(self.variance[1]), _lib.ptr(out), _lib.ptr(counts), _lib.ptr(kept),
-                                           _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+            _lib.check(Lb.fdt_detect_heads_ex(ld, cd, dt, fh, fw, nm, L, _lib.ptr(pri), num, int(self.top_k), int(self.nms_top_k),
+                                              float(self.conf_thresh), float(self.nms_thresh), float(self.variance[0]),
+                                              float(self.variance[1]), _lib.ptr(out), _lib.ptr(counts), _lib.ptr(kept),
+                                              _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
         del keep
         return (out, counts, kept) if return_aux else out
 

@@ -8,7 +8,7 @@ import torch.nn as nn
 
 from ... import _lib
 from ...data import face as cfg
-from ..functions.heads import _level_args, _map_grads
+from ..functions.heads import _head_args, _map_grads, map_descs
 
 
 def pack_targets(targets, device):
@@ -87,7 +87,7 @@ class _MultiBoxLossHeadsFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, priors, gt, gt_off, total_gt, threshold, negpos_ratio, bipartite, variance, neg_max, L, *maps):
-        dev, B, N, (conf, loc), (lp, cp, fh, fw, nm, _) = _level_args(maps[:L], maps[L:], neg_max)
+        dev, B, N, (conf, loc), (ld, cd, dt, fh, fw, nm, _) = _head_args(maps[:L], maps[L:], neg_max)
         pri = _lib.dev_f32(priors, dev)
         if pri.dim() != 2 or pri.size(1) != 4 or pri.size(0) != N:
             raise ValueError(f"MultiBoxLoss.forward_heads: priors must be [{N},4] (one per map position), got {tuple(pri.shape)}")
@@ -99,33 +99,31 @@ class _MultiBoxLossHeadsFn(torch.autograd.Function):
         with torch.cuda.device(dev):
             lib = _lib.lib()
             ws = _lib.workspace(lib.fdt_multibox_workspace_bytes(B, N, 2, total_gt), dev, "multibox")
-            _lib.check(lib.fdt_multibox_loss_forward_heads(
-                lp, cp, fh, fw, nm, L, _lib.ptr(pri), _lib.ptr(gt), _lib.ptr(gt_off), total_gt, B,
+            _lib.check(lib.fdt_multibox_loss_forward_heads_ex(
+                ld, cd, dt, fh, fw, nm, L, _lib.ptr(pri), _lib.ptr(gt), _lib.ptr(gt_off), total_gt, B,
                 float(threshold), int(negpos_ratio), int(bool(bipartite)), float(variance[0]), float(variance[1]),
                 _lib.ptr(losses), _lib.ptr(norm), _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), None,
                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
         ctx.save_for_backward(loc_t, conf_t, sel, norm, *loc, *conf)
-        ctx.level = (fh, fw, nm, L, B, dev)
+        ctx.level = (fh, fw, nm, L, B, dev, dt)
         ctx.mark_non_differentiable(loc_t, conf_t, sel)
         return losses[0].clone(), losses[1].clone(), loc_t, conf_t, sel
 
     @staticmethod
     def backward(ctx, g_l, g_c, *_):
-        fh, fw, nm, L, B, dev = ctx.level
+        fh, fw, nm, L, B, dev, dt = ctx.level
         loc_t, conf_t, sel, norm, *maps = ctx.saved_tensors
         loc, conf = maps[:L], maps[L:]
         need_loc, need_conf = any(ctx.needs_input_grad[10:10 + L]), any(ctx.needs_input_grad[10 + L:])
-        gl_maps, glp = _map_grads(loc, need_loc, dev)
-        gc_maps, gcp = _map_grads(conf, need_conf, dev)
+        gl_maps, gld = _map_grads(loc, need_loc)
+        gc_maps, gcd = _map_grads(conf, need_conf)
         zero = torch.zeros((), dtype=torch.float32, device=dev)
         gl = zero if g_l is None else g_l.detach().to(device=dev, dtype=torch.float32).contiguous()
         gc = zero if g_c is None else g_c.detach().to(device=dev, dtype=torch.float32).contiguous()
-        lp = (C.c_void_p * L)(*[m.data_ptr() for m in loc])
-        cp = (C.c_void_p * L)(*[m.data_ptr() for m in conf])
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().fdt_multibox_loss_backward_heads_dev(
-                lp, cp, fh, fw, nm, L, _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), _lib.ptr(norm),
-                _lib.ptr(gl), _lib.ptr(gc), B, glp, gcp, _lib.stream_ptr()))
+            _lib.check(_lib.lib().fdt_multibox_loss_backward_heads_dev_ex(
+                map_descs(loc), map_descs(conf), dt, fh, fw, nm, L, _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), _lib.ptr(norm),
+                _lib.ptr(gl), _lib.ptr(gc), B, gld, gcd, _lib.stream_ptr()))
         return (None,) * 10 + (*(gl_maps or [None] * L), *(gc_maps or [None] * L))
 
 

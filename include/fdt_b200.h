@@ -239,7 +239,22 @@ int fdt_detect_gather_store(const float *loc, const float *conf, const float *pr
  * softmax, the training path keeps raw logits).  fdt_detect_heads == fdt_heads_to_loc_conf(softmax) + fdt_detect with
  * nothing materialised: the threshold kernel reads the conf maps (max-in-out + softmax fused), NMS gathers the loc rows
  * it decodes from the loc maps.  Softmax: exp(x - max) in fp64 rounded once, fp32 sum and IEEE division.
- * Workspace of fdt_detect_heads: fdt_detect_workspace_bytes(B, N, 2).  Limit: n_levels <= 8. */
+ * Workspace of fdt_detect_heads: fdt_detect_workspace_bytes(B, N, 2).  Limit: n_levels <= 8.
+ *
+ * Mixed precision and channels_last: the `_ex` entries take each map as a descriptor -- element (b, ch, y, x) of a level is
+ * data[b * batch_stride + ch * channel_stride + (y * W + x) * pixel_stride], strides in elements, all > 0 -- and one element type
+ * for every map of the call (FDT_DTYPE_*).  Dense NCHW is (4*H*W, H*W, 1), dense channels_last (NHWC in memory) (4*H*W, 1, 4).
+ * The kernels read the maps in place and widen each element to fp32 (exact), so every output is bit-identical to the entry without
+ * `_ex` on the maps converted to fp32 NCHW.  Where a prior's four channels are adjacent and their address is a multiple of four
+ * elements, they are read with one vector load.  Gradient maps (fdt_head_grad_map) have the maps' element type and their own strides;
+ * a gradient is computed in fp32 as for fp32 maps and rounded to the element type (round to nearest even, overflow to +-inf).
+ * An unknown dtype, a null `data` of a map the call reads or writes, a stride <= 0 or a `data` not aligned to the element size is
+ * FDT_E_INVALID, checked before any CUDA call.  The entries without `_ex` are these with fp32 dense-NCHW descriptors. */
+#define FDT_DTYPE_F32  0
+#define FDT_DTYPE_BF16 1
+#define FDT_DTYPE_F16  2
+typedef struct { const void *data; int64_t batch_stride, channel_stride, pixel_stride; } fdt_head_map;
+typedef struct { void *data; int64_t batch_stride, channel_stride, pixel_stride; } fdt_head_grad_map;
 int fdt_heads_to_loc_conf(const float *const *loc_maps_h, const float *const *conf_maps_h,
                           const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, int B, int softmax,
                           float *loc_out, float *conf_out, fdt_stream_t stream);
@@ -247,6 +262,13 @@ int fdt_detect_heads(const float *const *loc_maps_h, const float *const *conf_ma
                      const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, const float *priors,
                      int B, int top_k, int nms_top_k, float conf_thresh, float nms_thresh, float var0, float var1,
                      float *out, int32_t *counts, int64_t *kept_prior, void *ws, size_t ws_bytes, fdt_stream_t stream);
+int fdt_heads_to_loc_conf_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype,
+                             const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, int B, int softmax,
+                             float *loc_out, float *conf_out, fdt_stream_t stream);
+int fdt_detect_heads_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype,
+                        const int *f_h, const int *f_w, const int *neg_max_h, int n_levels, const float *priors,
+                        int B, int top_k, int nms_top_k, float conf_thresh, float nms_thresh, float var0, float var1,
+                        float *out, int32_t *counts, int64_t *kept_prior, void *ws, size_t ws_bytes, fdt_stream_t stream);
 
 /* Diagnostics (FDT_K3_PROFILE=1): per-phase clock64 deltas of CTA 0 of the last fdt_detect_sort_nms / fdt_nms launch. */
 int fdt_debug_k3_profile(long long *out1024_h);  /* [0..31] phases of CTA 0, [64..319] cycles per CTA, [320..575] rounds*1e5 + k per CTA, [640..767] phase-B per warp */
@@ -319,7 +341,8 @@ int fdt_multibox_loss_backward_dev(const float *loc, const float *conf, const fl
                                    int B, int64_t N, int C, float *grad_loc, float *grad_conf, fdt_stream_t stream);
 
 /* ---- training from head maps (SURVEY 8f rank 1; replaces pyramid.py:291-309 + MyTrain_repo.py:170-171 and their autograd backward)
- * Map arguments as fdt_heads_to_loc_conf (HOST arrays of n_levels DEVICE pointers, NCHW [B,4,H_l,W_l]); N = sum H_l*W_l, C = 2.
+ * Map arguments as fdt_heads_to_loc_conf (HOST arrays of n_levels DEVICE pointers, NCHW [B,4,H_l,W_l]; the `_ex` entries: HOST arrays
+ * of descriptors, any element type and layout fdt_heads_to_loc_conf_ex accepts); N = sum H_l*W_l, C = 2.
  * Gradient maps have the maps' layout.  The gradient of a max-reduced logit goes to the channel torch's max(dim) backward picks: the
  * first NaN of the three channels if there is one, else the lowest channel equal to their maximum (-0.0 == +0.0); the other two
  * channels of the three receive +0.0.
@@ -343,6 +366,21 @@ int fdt_multibox_loss_backward_heads_dev(const float *const *loc_maps_h, const f
                                          const int64_t *conf_t, const uint8_t *sel, const float *norm, const float *g_l_dev,
                                          const float *g_c_dev, int B, float *const *grad_loc_maps_h,
                                          float *const *grad_conf_maps_h, fdt_stream_t stream);
+/* the same on map descriptors (see fdt_heads_to_loc_conf_ex) */
+int fdt_heads_to_loc_conf_backward_ex(const fdt_head_map *conf_maps_h, int dtype, const int *f_h, const int *f_w, const int *neg_max_h,
+                                      int n_levels, int B, int softmax, const float *grad_loc, const float *grad_conf,
+                                      const fdt_head_grad_map *grad_loc_maps_h, const fdt_head_grad_map *grad_conf_maps_h,
+                                      fdt_stream_t stream);
+int fdt_multibox_loss_forward_heads_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype, const int *f_h,
+                                       const int *f_w, const int *neg_max_h, int n_levels, const float *priors, const float *gt,
+                                       const int64_t *gt_off, int64_t total_gt, int B, float threshold, int negpos_ratio, int bipartite,
+                                       float var0, float var1, float *losses, float *norm, float *loc_t, int64_t *conf_t, uint8_t *sel,
+                                       float *loss_c_all, void *ws, size_t ws_bytes, fdt_stream_t stream);
+int fdt_multibox_loss_backward_heads_dev_ex(const fdt_head_map *loc_maps_h, const fdt_head_map *conf_maps_h, int dtype, const int *f_h,
+                                            const int *f_w, const int *neg_max_h, int n_levels, const float *loc_t,
+                                            const int64_t *conf_t, const uint8_t *sel, const float *norm, const float *g_l_dev,
+                                            const float *g_c_dev, int B, const fdt_head_grad_map *grad_loc_maps_h,
+                                            const fdt_head_grad_map *grad_conf_maps_h, fdt_stream_t stream);
 
 /* ---- T2  IoU tracker association  (iouTracke_cal.py:126-155 loop, :174-176 flush) ----------------
  * dets[total,5] float64 rows [x1,y1,x2,y2,score]; frame_off[F+1] int64 (device); frames are 1-based in
