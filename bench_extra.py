@@ -12,6 +12,7 @@
     python bench_extra.py heads      # SURVEY 8f rank 1: Detect straight from the per-level NCHW head maps, B=64 @640^2
     python bench_extra.py heads_train # SURVEY 8f rank 1: MultiBoxLoss (+ backward) straight from the head maps, B=32 @640^2 (config 3)
     python bench_extra.py match_mine # fdt_match_encode and fdt_hard_negative_mine on their own (box_utils.match_*, DataEncoder.encode)
+    python bench_extra.py flat_amp   # bf16 / fp16 flat loc / conf read in place by Detect, Detect.submit and MultiBoxLoss vs converted
     python bench_extra.py track_stream # online tracker: V in {1, 64, 148} streams x 2,000 config-4 frames, one frame per stream per
                                      # step, vs the offline tracker per video; Detect B=64 @640^2 + step_detections vs Detect alone
 
@@ -667,6 +668,123 @@ def heads_amp():
                                    "forward_bytes": B * N * (8 * esz + 16 + 8 + 1)}
     print(json.dumps({"workload": "head maps as the network wrote them (bf16 / fp16, NCHW / channels_last) vs converted to fp32 NCHW; "
                       "Detect B=64 and MultiBoxLoss B=32 @640x640", **card(), "results": res}))
+
+
+def flat_amp():
+    """Flat loc[B,N,4] / conf[B,N,C] of 16-bit dtypes read in place vs the conversion path (loc.float(), conf.float() before the call,
+    which is what every non-fp32 input cost before).  Rows: Detect B=64 @640x640 isolated and back to back for fp32, (bf16 loc, fp32
+    conf) = inference under autocast, bf16 / bf16 and fp16 / fp16 (plus `fp32_same_values`: the fp32 call on the 16-bit values converted
+    before timing, which separates what reading 16-bit data costs from what the coarser scores cost); Detect B=512 @1024x1024 bf16 (more lists than SMs: K2 + k_sort_nms);
+    Detect.submit streamed from pinned host tensors, fp16 against fp32 (two batches in flight); MultiBoxLoss B=32 @640x640 bf16 forward
+    and forward + backward through the autograd module, both matchers.  `equal` = the in-place result is bit-identical to the
+    conversion path's in this run.  tie_runs: per dtype, the images whose nms_top_k best candidates hold a run of more than 512 equal
+    scores (a bucket too large for k_sort_nms' per-window ranking: its bitonic fallback) -- a count from the inputs, not a kernel
+    counter."""
+    from fdt_b200.layers import Detect, MultiBoxLoss
+    res = {}
+
+    def b2b(call, n=50):
+        for i in range(8):
+            call(i)
+        torch.cuda.synchronize()
+        blocks = []
+        for _ in range(5):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            torch.cuda._sleep(2_000_000)
+            e0.record()
+            for i in range(n):
+                call(i)
+            e1.record()
+            torch.cuda.synchronize()
+            blocks.append(e0.elapsed_time(e1) / n)
+        return float(np.median(blocks))
+
+    def tie_runs(conf, k=5000, run=512):
+        s = conf[..., 1].float()
+        top = torch.topk(torch.where(s > 0.05, s, torch.full_like(s, -1.0)), k, dim=1).values
+        n = 0
+        for row in top:
+            row = row[row > 0.05]
+            if row.numel() and int(torch.unique(row, return_counts=True)[1].max()) > run:
+                n += 1
+        return n
+
+    def detect_rows(B, w, prefix, cases, n_b2b=50):
+        pri = torch.from_numpy(synth.priors_numpy(w, w)).cuda()
+        raw = [synth.detect_inputs(B, synth.priors_numpy(w, w), 7070 + i) for i in range(2)]
+        det = Detect(2, 0, 750, 0.05, 0.3)
+        for name, ldt, cdt in cases:
+            sets = [(torch.from_numpy(l).to(ldt).cuda(), torch.from_numpy(c).to(cdt).cuda()) for l, c in raw]
+            up = [(l.float(), c.float()) for l, c in sets]
+            row = {}
+            for mode in ("converted", "in_place", "fp32_same_values"):
+                def call(i, mode=mode):
+                    l, c = sets[i % 2]
+                    if mode == "fp32_same_values":          # the fp32 call on the rounded values, converted before timing
+                        return det(*up[i % 2], pri)
+                    return det(l.float(), c.float(), pri) if mode == "converted" else det(l, c, pri)
+                row[mode + "_isolated_ms"], _ = timed(lambda: call(0))
+                row[mode + "_back_to_back_ms"] = b2b(call, n_b2b)
+            a = det(*sets[0], pri, return_aux=True)
+            b = det(sets[0][0].float(), sets[0][1].float(), pri, return_aux=True)
+            row["equal"] = all(torch.equal(x.view(torch.uint8), y.view(torch.uint8)) for x, y in zip(a, b))
+            row["tie_runs_over_512"] = tie_runs(sets[0][1])
+            res[prefix + name] = row
+    F32, BF, HF = torch.float32, torch.bfloat16, torch.float16
+    detect_rows(64, 640, "detect_b64_640_", [("fp32", F32, F32), ("bf16loc_fp32conf", BF, F32), ("bf16", BF, BF), ("fp16", HF, HF)])
+    detect_rows(512, 1024, "detect_b512_1024_", [("bf16", BF, BF)], n_b2b=10)
+    # ---- Detect.submit from pinned host tensors, two batches in flight (the host path is bound by the conf copy)
+    B = 64
+    pri_h = torch.from_numpy(synth.priors_numpy(640, 640))
+    l0, c0 = synth.detect_inputs(B, synth.priors_numpy(640, 640), 7171)
+    det = Detect(2, 0, 750, 0.05, 0.3)
+    for name, dt in (("fp32", F32), ("fp16", HF)):
+        l, c = torch.from_numpy(l0).to(dt).pin_memory(), torch.from_numpy(c0).to(dt).pin_memory()
+        out = det.submit(l, c, pri_h).result()
+        for _ in range(4):
+            det.submit(l, c, pri_h).result()
+        n, t0 = 40, time.perf_counter()
+        pend = [det.submit(l, c, pri_h)]
+        for _ in range(n - 1):
+            pend.append(det.submit(l, c, pri_h))
+            pend.pop(0).result()
+        pend.pop(0).result()
+        dtm = (time.perf_counter() - t0) / n * 1e3
+        up = det.submit(l.float(), c.float(), pri_h).result()
+        res["detect_submit_b64_640_pinned_" + name] = {"ms_per_batch": dtm, "conf_bytes": B * c.shape[1] * 2 * c.element_size(),
+                                                       "equal": bool(torch.equal(out.view(torch.uint8), up.view(torch.uint8)))}
+    # ---- MultiBoxLoss B = 32, bf16 (training under autocast), through the autograd module
+    B = 32
+    pri = torch.from_numpy(synth.priors_numpy(640, 640)).cuda()
+    l0, c0, targets = synth.multibox_inputs(B, synth.priors_numpy(640, 640), 3030, 0, 200)
+    tg = [torch.from_numpy(t).cuda() for t in targets]
+    for bip in (False, True):
+        crit = MultiBoxLoss(2, 0.35, True, 0, True, 3, 0.35, False, bipartite=bip)
+        loc = torch.from_numpy(l0).to(BF).cuda().requires_grad_(True)
+        conf = torch.from_numpy(c0).to(BF).cuda().requires_grad_(True)
+        row, got = {}, {}
+        for mode in ("converted", "in_place"):
+            def args(mode=mode):
+                return (loc.float(), conf.float(), pri) if mode == "converted" else (loc, conf, pri)
+
+            def fwd():
+                with torch.no_grad():
+                    return crit(args(), tg)
+
+            def fwd_bwd():
+                loc.grad = conf.grad = None
+                ll, lc = crit(args(), tg)
+                (ll + lc).backward()
+                return ll, lc
+            ll, lc = fwd_bwd()
+            got[mode] = (float(ll.detach()), float(lc.detach()), loc.grad.view(torch.int16).clone(), conf.grad.view(torch.int16).clone())
+            row[mode + "_forward_ms"], _ = timed(fwd)
+            row[mode + "_forward_backward_ms"], _ = timed(fwd_bwd)
+        a, b = got["converted"], got["in_place"]
+        row["equal"] = a[:2] == b[:2] and torch.equal(a[2], b[2]) and torch.equal(a[3], b[3])
+        res["loss_b32_640_bf16_" + ("bipartite" if bip else "default")] = row
+    print(json.dumps({"workload": "flat loc / conf in bf16 / fp16 read in place vs converted to fp32 first: Detect B=64 @640^2 and "
+                      "B=512 @1024^2, Detect.submit from pinned host tensors, MultiBoxLoss B=32 @640^2", **card(), "results": res}))
 
 
 def card():

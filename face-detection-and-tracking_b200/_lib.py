@@ -71,6 +71,10 @@ SIGNATURES = {
     "fdt_detect_host": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp]),
     "fdt_detect_host_submit": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp, C.POINTER(C.c_uint64)]),
     "fdt_detect_host_wait": (_i, [_vp, C.c_uint64]),
+    "fdt_detect_ex": (_i, [_vp, _i, _vp, _i, _vp, _i, _i64, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_detect_host_ex": (_i, [_vp, _vp, _i, _vp, _i, _vp, _i, _i64, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp]),
+    "fdt_detect_host_submit_ex": (_i, [_vp, _vp, _i, _vp, _i, _vp, _i, _i64, _i, _i, _i, _f, _f, _f, _f, _vp, _vp, _vp,
+                                       C.POINTER(C.c_uint64)]),
     "fdt_match_workspace_bytes": (_sz, [_i, _i64, _i64]),
     "fdt_match_encode": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _f, _f, _f, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fdt_mine_workspace_bytes": (_sz, [_i, _i64]),
@@ -80,6 +84,9 @@ SIGNATURES = {
                                        _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "fdt_multibox_loss_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _f, _f, _i, _i64, _i, _vp, _vp, _vp]),
     "fdt_multibox_loss_backward_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
+    "fdt_multibox_loss_forward_ex": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _i64, _i, _i64, _i, _f, _i, _i, _f, _f,
+                                          _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "fdt_multibox_loss_backward_dev_ex": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp]),
     "fdt_heads_to_loc_conf_backward": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "fdt_multibox_loss_forward_heads": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i64, _i, _f, _i, _i, _f, _f,
                                              _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -235,3 +242,20 @@ def dev_f32(t: torch.Tensor, device: torch.device) -> torch.Tensor:
     if t.data_ptr() % 16:
         t = t.clone()
     return t
+
+
+FDT_DTYPE_F32, FDT_DTYPE_BF16, FDT_DTYPE_F16 = 0, 1, 2
+_DTYPE16 = {torch.bfloat16: FDT_DTYPE_BF16, torch.float16: FDT_DTYPE_F16}
+
+
+def flat_input(t: torch.Tensor, device: torch.device):
+    """A flat loc / conf tensor as the `_ex` entries take it -> (tensor, FDT_DTYPE_*).  A contiguous bf16 / fp16 tensor on `device` is
+    passed in place (any storage offset: the kernels take any element-aligned address); everything else becomes what it always
+    became: dev_f32 on a CUDA device, a contiguous fp32 copy on the host."""
+    t = t.detach()
+    code = _DTYPE16.get(t.dtype)
+    if code is not None and t.device == device and t.is_contiguous():
+        return t, code
+    if device.type == "cpu":
+        return t.to(torch.float32).contiguous(), FDT_DTYPE_F32
+    return dev_f32(t, device), FDT_DTYPE_F32

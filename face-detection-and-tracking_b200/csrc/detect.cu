@@ -356,7 +356,20 @@ k_heads_threshold_compact(const HeadLevels hl, const int64_t N, const float thr,
     }
 }
 
-// SRC 0: conf[B,N,C] with C > 2; 1: conf[B,N,2]
+// score of prior i, class cl, of a 16-bit (bf16 / fp16) conf[B,N,C], widened to fp32 (exact); row0 = element (b, 0, 0).  pair: C == 2 and
+// row0 4-byte aligned, so the (background, face) pair of a prior is one 32-bit word whose high half is the face score -- bf16 widens
+// with one AND.
+__device__ __forceinline__ float conf16_score(const unsigned short *row0, const int64_t i, const int C, const int cl, const int dtype,
+                                              const bool pair)
+{
+    if (pair) {
+        const unsigned w = __ldg(reinterpret_cast<const unsigned *>(row0) + i);
+        return dtype == FDT_DTYPE_BF16 ? __uint_as_float(w & 0xffff0000u) : __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+    }
+    return head_widen16(__ldg(row0 + i * C + cl), dtype);
+}
+
+// SRC 0: conf[B,N,C] with C > 2; 1: conf[B,N,2]; 2: 16-bit conf[B,N,C] of element type hl.dtype (hl.vec bit 0: conf16_score's pair)
 #ifndef FDT_K2_MINBLOCKS
 #define FDT_K2_MINBLOCKS 6
 #endif
@@ -385,6 +398,25 @@ k_threshold_compact(const float *__restrict__ conf, const HeadLevels hl, int64_t
         unsigned bal[K2_PER_THREAD];
         int wtotal = 0;
         unsigned kmx = 0u, kmnv = 0u;                    // max key and max ~key (= ~min key) of this thread's candidates
+        if constexpr (SRC == 2) {
+            // the dtype / pair choice is uniform: taken once per tile, not per prior (a branch per load cost a third of this kernel)
+            const unsigned short *c16 = reinterpret_cast<const unsigned short *>(conf) + (int64_t)b * N * C;
+            const bool bf = hl.dtype == FDT_DTYPE_BF16;
+            if (hl.vec & 1u) {
+#pragma unroll
+                for (int u = 0; u < K2_PER_THREAD; ++u) {
+                    const int64_t p = base + u * K2_THREADS + tid;
+                    const unsigned w = p < N ? __ldg(reinterpret_cast<const unsigned *>(c16) + p) : 0u;
+                    sc[u] = bf ? __uint_as_float(w & 0xffff0000u) : __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+                }
+            } else {
+#pragma unroll
+                for (int u = 0; u < K2_PER_THREAD; ++u) {
+                    const int64_t p = base + u * K2_THREADS + tid;
+                    sc[u] = p < N ? head_widen16(__ldg(c16 + p * C + cl), hl.dtype) : 0.0f;
+                }
+            }
+        } else {
 #pragma unroll
         for (int u = 0; u < K2_PER_THREAD; ++u) {        // the tile's loads are in flight before anything below waits
             const int64_t p = base + u * K2_THREADS + tid;
@@ -394,6 +426,7 @@ k_threshold_compact(const float *__restrict__ conf, const HeadLevels hl, int64_t
                 else s = __ldg(cb + p * C + cl);
             }
             sc[u] = s;
+        }
         }
         if (cl == 1) {
             my_seq = detect_call_seq(S, &s_seq);
@@ -529,6 +562,8 @@ struct SortNmsParams {
     HeadLevels hl;              // per-level NCHW loc maps (MODE_DETECT with loc == null)
     long long *prof;            // diagnostics: per-phase clock64 of CTA 0 (null unless FDT_K3_PROFILE=1 / 2)
     int prof_all;               // FDT_K3_PROFILE=2: every CTA of every launch ADDS its phase clocks (steady-state averages; [30] counts CTAs)
+    int conf_dtype;             // FUSED with HT = 1: FDT_DTYPE_* of `conf` (the pointer then addresses elements of that type)
+    int conf_pair;              // ... 16-bit, C == 2, 4-byte aligned: conf16_score's pair load
 };
 
 // "i (kept, higher score) suppresses j": box_utils.py:322-339, union = (area_j - inter) + area_i,
@@ -783,7 +818,9 @@ __device__ __forceinline__ void csr_scan(int *a, int *s_warp)
 #define K3_BOUNDS __launch_bounds__(K3_THREADS, 1)
 #endif
 // HT = 1: MODE_DETECT with the loc rows gathered from head maps other than fp32 dense NCHW (HEAD_ANY, heads.cuh): in the
-// instantiations above their loads and widening would cost the 64-register kernel extra spill traffic
+// instantiations above their loads and widening would cost the 64-register kernel extra spill traffic.  A flat loc[B,N,4] of a
+// 16-bit type is such a map (one level, hw = N, strides (4N, 1, 4)).  FUSED with HT = 1 is the fused kernel for flat inputs of which
+// at least one is 16-bit: loc through its one-level map (any element type), conf of element type P.conf_dtype widened as it is read.
 template <int MODE, int CL, bool FUSED, int HT = 0>
 __global__ void K3_BOUNDS
 k_sort_nms(const SortNmsParams P)
@@ -953,6 +990,12 @@ k_sort_nms(const SortNmsParams P)
         uint64_t *wq = reinterpret_cast<uint64_t *>(smem + SM_SEGS) + warp * WQ_CAP;
         const int Nn = (int)P.N, Cc = P.C;
         auto key_of = [&](const float sc, const int i) -> uint64_t { return ((uint64_t)fdt_float_key(sc) << 32) | (uint32_t)i; };
+        // HT = 1: score of prior i of the list, of element type P.conf_dtype, widened to fp32 (exact) before any compare
+        auto conf_any = [&](const int i) -> float {
+            if (P.conf_dtype == FDT_DTYPE_F32) return __ldg(reinterpret_cast<const float *>(P.conf) + ((int64_t)b * Nn + i) * Cc + cl);
+            return conf16_score(reinterpret_cast<const unsigned short *>(P.conf) + (int64_t)b * Nn * Cc, i, Cc, cl, P.conf_dtype,
+                                P.conf_pair != 0);
+        };
         auto for_each_key = [&](auto &&body) {
             if (FUSED) {
                 if (!scanned) {
@@ -971,7 +1014,27 @@ k_sort_nms(const SortNmsParams P)
                     auto load_group = [&](const int g) {
                         const int i0 = tid + g * UG * K3_THREADS;
                         const bool whole = (g + 1) * UG * K3_THREADS <= Nn;                  // (uniform) no prior of the group is past the row
-                        if (Cc == 2) {                                                       // (addresses fold into the load immediates)
+                        if constexpr (HT == 1) {
+                            if (P.conf_pair) {          // (uniform) the prior's 32-bit (background, face) word, addresses folded
+                                const unsigned *w0 = reinterpret_cast<const unsigned *>(P.conf) + (int64_t)b * Nn + i0;
+                                const bool bf = P.conf_dtype == FDT_DTYPE_BF16;
+#pragma unroll
+                                for (int u = 0; u < UG; ++u) {
+                                    const unsigned w = (whole || i0 + u * K3_THREADS < Nn) ? __ldg(w0 + u * K3_THREADS) : 0x7fc00000u;
+                                    sv[g][u] = bf ? __uint_as_float(w & 0xffff0000u) : __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+                                }
+                            } else if (P.conf_dtype == FDT_DTYPE_F32 && Cc == 2) {     // (uniform) fp32 conf beside a 16-bit loc
+                                const float *p0 = reinterpret_cast<const float *>(P.conf) + ((int64_t)b * Nn + i0) * 2 + cl;
+#pragma unroll
+                                for (int u = 0; u < UG; ++u) sv[g][u] = (whole || i0 + u * K3_THREADS < Nn) ? __ldg(p0 + 2 * u * K3_THREADS) : qnan;
+                            } else {
+#pragma unroll
+                                for (int u = 0; u < UG; ++u) {
+                                    const int i = i0 + u * K3_THREADS;
+                                    sv[g][u] = (whole || i < Nn) ? conf_any(i) : qnan;
+                                }
+                            }
+                        } else if (Cc == 2) {                                                // (addresses fold into the load immediates)
                             const float *p0 = crow + 2 * i0;
                             if (whole) {
 #pragma unroll
@@ -1031,7 +1094,9 @@ k_sort_nms(const SortNmsParams P)
                 for (int e = lane; e < wq_n; e += 32) body(wq[e]);
                 // in place (re-read, L2): the whole first round of a warp whose queue overflowed, and every prior beyond it
                 for (int i = (wq_ovf ? 0 : U * K3_THREADS) + tid; i < Nn; i += K3_THREADS) {
-                    const float sc = __ldg(crow + (int64_t)i * Cc);
+                    float sc;
+                    if constexpr (HT == 1) sc = conf_any(i);
+                    else sc = __ldg(crow + (int64_t)i * Cc);
                     if (sc > cthr) body(key_of(sc, i));
                 }
             } else if (cached) {
@@ -1120,7 +1185,9 @@ k_sort_nms(const SortNmsParams P)
                         uint64_t key;
                         bool cand = true;
                         if (FUSED) {
-                            const float sc = __ldg(crow + (int64_t)i * P.C);
+                            float sc;
+                            if constexpr (HT == 1) sc = conf_any(i);
+                            else sc = __ldg(crow + (int64_t)i * P.C);
                             cand = sc > cthr;
                             key = ((uint64_t)fdt_float_key(sc) << 32) | (uint32_t)i;
                         } else key = __ldcg(gkeys + i);
@@ -1807,9 +1874,12 @@ int launch_sort_nms(SortNmsParams &P, int lists, int kcap, void *kept_ws, size_t
         ++na;
     }
     cfg.attrs = attr; cfg.numAttrs = na;
-    static FuncAttrCache cache_cl, cache_1, cache_f, cache_cl_any, cache_1_any;
+    static FuncAttrCache cache_cl, cache_1, cache_f, cache_cl_any, cache_1_any, cache_f_any;
     const bool head_any = MODE == MODE_DETECT && P.loc == nullptr && !P.hl.f32_nchw;
-    if (head_any && cluster) {
+    if (fused && (P.loc == nullptr || P.conf_dtype != FDT_DTYPE_F32)) {         // flat inputs, at least one of them 16-bit
+        int rc = ensure_dyn_smem(k_sort_nms<MODE_DETECT, 1, true, 1>, cache_f_any, sp.total); if (rc != FDT_OK) return rc;
+        FDT_CUDA(cudaLaunchKernelEx(&cfg, k_sort_nms<MODE_DETECT, 1, true, 1>, P));
+    } else if (head_any && cluster) {
         int rc = ensure_dyn_smem(k_sort_nms<MODE_DETECT, 2, false, 1>, cache_cl_any, sp.total); if (rc != FDT_OK) return rc;
         FDT_CUDA(cudaLaunchKernelEx(&cfg, k_sort_nms<MODE_DETECT, 2, false, 1>, P));
     } else if (head_any) {
@@ -1923,15 +1993,17 @@ static int detect_check_common(const char *who, int B, int64_t N, int C, const v
 // them); the stage entry point does not know them and serialises instead.
 static int threshold_compact_impl(const float *conf, const HeadLevels *heads, int B, int64_t N, int C, float conf_thresh,
                                   void *ws, size_t ws_bytes, fdt_stream_t stream,
-                                  const void *out0, const void *out1, const void *out2, int serialize, bool begin_only = false)
+                                  const void *out0, const void *out1, const void *out2, int serialize, bool begin_only = false,
+                                  int conf_dtype = FDT_DTYPE_F32)
 {
     cudaStream_t st = (cudaStream_t)stream;
     int rc = detect_check_common("fdt_detect_threshold_compact", B, N, C, ws, ws_bytes);
     if (rc != FDT_OK) return rc;
     const int lists = B * (C - 1);
     if (lists == 0 || N == 0) return FDT_OK;
-    FDT_REQUIRE(heads || (conf && fdt_aligned(conf, 4)), FDT_E_INVALID, "fdt_detect: conf null or not 4-byte aligned");
-    FDT_REQUIRE(heads || begin_only || C != 2 || fdt_aligned(conf, 8), FDT_E_INVALID, "fdt_detect_threshold_compact: conf not 8-byte aligned");
+    const bool c16 = conf_dtype != FDT_DTYPE_F32;
+    FDT_REQUIRE(heads || (conf && fdt_aligned(conf, c16 ? 2 : 4)), FDT_E_INVALID, "fdt_detect: conf null or not aligned to its elements");
+    FDT_REQUIRE(heads || begin_only || c16 || C != 2 || fdt_aligned(conf, 8), FDT_E_INVALID, "fdt_detect_threshold_compact: conf not 8-byte aligned");
     const DetectWsPlan w = detect_ws_plan(B, N, C);
     const DetectSlots S = detect_slots(ws, ws_bytes, w);
     long long *prof = nullptr;
@@ -1967,6 +2039,11 @@ static int threshold_compact_impl(const float *conf, const HeadLevels *heads, in
             else if (conf_thresh >= 1.0f - 1e-4f) dcut = 9.0f;          // sigmoid(9) < 1 - 1e-4: nothing at or below can pass
             if (hl.f32_nchw) FDT_CUDA(cudaLaunchKernelEx(&cfg, k_heads_threshold_compact<HEAD_F32_NCHW>, hl, N_, conf_thresh, dcut, S, prof));
             else             FDT_CUDA(cudaLaunchKernelEx(&cfg, k_heads_threshold_compact<HEAD_ANY>, hl, N_, conf_thresh, dcut, S, prof));
+        }
+        else if (c16) {
+            hl.dtype = conf_dtype;
+            hl.vec = (C == 2 && fdt_aligned(conf, 4)) ? 1u : 0u;
+            FDT_CUDA(cudaLaunchKernelEx(&cfg, k_threshold_compact<2>, conf, hl, N_, C, conf_thresh, S, prof));
         }
         else if (C == 2) FDT_CUDA(cudaLaunchKernelEx(&cfg, k_threshold_compact<1>, conf, hl, N_, C, conf_thresh, S, prof));
         else             FDT_CUDA(cudaLaunchKernelEx(&cfg, k_threshold_compact<0>, conf, hl, N_, C, conf_thresh, S, prof));
@@ -2021,8 +2098,10 @@ static int detect_sort_nms_impl(const float *loc, const HeadLevels *heads, const
                                 float nms_thresh, float var0, float var1,
                                 float *out, int32_t *counts, int64_t *kept_prior,
                                 const GatherArgs &G, void *ws, size_t ws_bytes, fdt_stream_t stream,
-                                const float *fused_conf = nullptr, float conf_thresh = 0.0f, unsigned flags = 0)
+                                const float *fused_conf = nullptr, float conf_thresh = 0.0f, unsigned flags = 0,
+                                int conf_dtype = FDT_DTYPE_F32, bool flat = false)
 {
+    // flat: `heads` describes a flat loc[B,N,4] (flat_loc_levels), and stage 1 was the flat K2 (its grid counts K2_TILE priors per block)
     cudaStream_t st = (cudaStream_t)stream;
     int rc = detect_check_common("fdt_detect_sort_nms", B, N, C, ws, ws_bytes);
     if (rc != FDT_OK) return rc;
@@ -2045,10 +2124,11 @@ static int detect_sort_nms_impl(const float *loc, const HeadLevels *heads, const
                 "fdt_detect: loc/priors null or not 16-byte aligned");
     const DetectWsPlan w = detect_ws_plan(B, N, C);
     SortNmsParams P{};
-    P.S = detect_slots(ws, ws_bytes, w); P.use_counters = 1; P.key_stride = N; P.k2_blocks = k2_grid_x(N, heads != nullptr) * B;
+    P.S = detect_slots(ws, ws_bytes, w); P.use_counters = 1; P.key_stride = N; P.k2_blocks = k2_grid_x(N, heads != nullptr && !flat) * B;
     P.loc = heads ? nullptr : loc; P.priors = priors; P.N = N; P.C = C;
     P.loc_prefetch = (!heads && !(flags & FDT_FLAG_LOC_HOST_MAPPED) && options().detect_prefetch.load() == 1) ? 1 : 0;
     P.conf = fused_conf; P.conf_thresh = conf_thresh;
+    P.conf_dtype = conf_dtype; P.conf_pair = conf_dtype != FDT_DTYPE_F32 && C == 2 && fdt_aligned(fused_conf, 4);
     if (heads) P.hl = *heads;
     P.nms_top_k = nms_top_k; P.max_keep = top_k < nms_top_k ? top_k : nms_top_k; P.top_k = top_k;
     P.nms_thresh = nms_thresh; P.v0 = var0; P.v1 = var1;
@@ -2071,20 +2151,59 @@ FDT_API int fdt_detect_sort_nms(const float *loc, const float *priors, int B, in
 
 // One whole Detect call: sequencing + (K2 +) k_sort_nms.  Plain `conf` input takes the fused kernel (no K2); head maps and
 // fdt_set_option("detect_fused", 0) take K2 + k_sort_nms.
-static int detect_call(const float *loc, const float *conf, const float *priors, int B, int64_t N, int C, int top_k, int nms_top_k,
+// a flat loc[B,N,4] as a one-level loc map (heads.cuh): hw = N, strides (4N, 1, 4), one vector load per row where aligned
+static HeadLevels flat_loc_levels(const void *loc, int64_t N, int dtype)
+{
+    HeadLevels hl{};
+    hl.L = 1;
+    hl.dtype = dtype;
+    hl.hw[0] = (int)N;
+    hl.loc[0] = HeadMap{loc, 4 * N, 1, 4};
+    for (int l = 1; l <= FDT_MAX_LEVELS; ++l) hl.off[l] = (int)N;
+    hl.vec = fdt_aligned(loc, (size_t)(4 * head_elem_bytes(dtype))) ? 1u << 8 : 0u;
+    return hl;
+}
+
+static int detect_call(const void *loc, const void *conf, const float *priors, int B, int64_t N, int C, int top_k, int nms_top_k,
                        float conf_thresh, float nms_thresh, float var0, float var1,
                        float *out, int32_t *counts, int64_t *kept_prior, const GatherArgs &G, const void *alias0,
-                       void *ws, size_t ws_bytes, fdt_stream_t stream, unsigned flags = 0)
+                       void *ws, size_t ws_bytes, fdt_stream_t stream, unsigned flags = 0,
+                       int loc_dtype = FDT_DTYPE_F32, int conf_dtype = FDT_DTYPE_F32)
 {
     // Fused pays when one wave of CTAs holds every list (what counts then is SM time per list, and consecutive calls fill the
     // other SMs); with several waves of lists the chip-wide K2 streams conf at a higher rate than 148 CTAs scanning their own rows,
     // and rows much longer than the per-warp candidate queues (34 x 1024 priors per round) would mostly be visited in place.
     const int want = options().detect_fused.load();
     const bool fused = want < 0 ? ((int64_t)B * (C - 1) <= FDT_NUM_SMS && N <= 40960) : want == 1;
-    int rc = threshold_compact_impl(conf, nullptr, B, N, C, conf_thresh, ws, ws_bytes, stream, alias0, counts, kept_prior, 0, fused);
+    // before anything is enqueued: a null loc read through its one-level map (16-bit inputs) would be gathered from address 0
+    FDT_REQUIRE(B <= 0 || N <= 0 || C < 2 || (loc && priors), FDT_E_INVALID, "fdt_detect: loc / priors is null");
+    const float *conf32 = (const float *)conf;
+    int rc = threshold_compact_impl(conf32, nullptr, B, N, C, conf_thresh, ws, ws_bytes, stream, alias0, counts, kept_prior, 0, fused,
+                                    conf_dtype);
     if (rc != FDT_OK) return rc;
-    return detect_sort_nms_impl(loc, nullptr, priors, B, N, C, top_k, nms_top_k, nms_thresh, var0, var1, out, counts, kept_prior,
-                                G, ws, ws_bytes, stream, fused ? conf : nullptr, conf_thresh, flags);
+    if (loc_dtype == FDT_DTYPE_F32 && conf_dtype == FDT_DTYPE_F32)
+        return detect_sort_nms_impl((const float *)loc, nullptr, priors, B, N, C, top_k, nms_top_k, nms_thresh, var0, var1, out, counts,
+                                    kept_prior, G, ws, ws_bytes, stream, fused ? conf32 : nullptr, conf_thresh, flags);
+    // 16-bit input(s): a 16-bit loc is gathered through its one-level map by the HT = 1 instantiations (fused or not); the fused kernel for
+    // 16-bit conf (k_sort_nms<MODE_DETECT, 1, true, 1>) reads loc through that map whatever its type.  An fp32 loc with K2 keeps P.loc.
+    const bool via_map = loc_dtype != FDT_DTYPE_F32 || fused;
+    const HeadLevels hl = flat_loc_levels(loc, N, loc_dtype);
+    return detect_sort_nms_impl((const float *)loc, via_map ? &hl : nullptr, priors, B, N, C, top_k, nms_top_k, nms_thresh, var0, var1,
+                                out, counts, kept_prior, G, ws, ws_bytes, stream, fused ? conf32 : nullptr, conf_thresh, flags,
+                                conf_dtype, true);
+}
+
+// The element types and alignments of flat loc / conf (checked before any CUDA call): FDT_DTYPE_*, each pointer aligned to its
+// elements, an fp32 loc to f32_loc_align bytes.  Null pointers are the caller's to refuse (each entry knows when it reads them).
+int fdt_flat_inputs_ok(const char *who, const void *loc, int loc_dtype, const void *conf, int conf_dtype, size_t f32_loc_align)
+{
+    for (int d : {loc_dtype, conf_dtype})
+        FDT_REQUIRE(d == FDT_DTYPE_F32 || d == FDT_DTYPE_BF16 || d == FDT_DTYPE_F16, FDT_E_INVALID, "%s: unknown dtype %d", who, d);
+    const size_t la = loc_dtype == FDT_DTYPE_F32 ? f32_loc_align : 2;
+    FDT_REQUIRE(!loc || fdt_aligned(loc, la), FDT_E_INVALID, "%s: loc is not aligned to %d bytes", who, (int)la);
+    FDT_REQUIRE(!conf || fdt_aligned(conf, (size_t)head_elem_bytes(conf_dtype)), FDT_E_INVALID, "%s: conf is not aligned to its elements",
+                who);
+    return FDT_OK;
 }
 
 // Destination side of the signalled gather: ends when every rank -- this one included -- has published `epoch` in this rank's signal
@@ -2178,14 +2297,26 @@ FDT_API int fdt_detect_gather_store(const float *loc, const float *conf, const f
                        n_dest, peer_signal_ptrs, world, rank, root, epoch, ring, image_offset, ws, ws_bytes, stream, false);
 }
 
-int fdt_detect_flags(const float *loc, const float *conf, const float *priors,
+int fdt_detect_flags(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *priors,
                      int B, int64_t N, int C, int top_k, int nms_top_k,
                      float conf_thresh, float nms_thresh, float var0, float var1,
                      float *out, int32_t *counts, int64_t *kept_prior,
                      void *ws, size_t ws_bytes, fdt_stream_t stream, unsigned flags)
 {
     return detect_call(loc, conf, priors, B, N, C, top_k, nms_top_k, conf_thresh, nms_thresh, var0, var1, out, counts, kept_prior,
-                       GatherArgs{}, out, ws, ws_bytes, stream, flags);
+                       GatherArgs{}, out, ws, ws_bytes, stream, flags, loc_dtype, conf_dtype);
+}
+
+FDT_API int fdt_detect_ex(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *priors,
+                          int B, int64_t N, int C, int top_k, int nms_top_k,
+                          float conf_thresh, float nms_thresh, float var0, float var1,
+                          float *out, int32_t *counts, int64_t *kept_prior,
+                          void *ws, size_t ws_bytes, fdt_stream_t stream)
+{
+    int rc = fdt_flat_inputs_ok("fdt_detect", loc, loc_dtype, conf, conf_dtype, 16);
+    if (rc != FDT_OK) return rc;
+    return fdt_detect_flags(loc, loc_dtype, conf, conf_dtype, priors, B, N, C, top_k, nms_top_k, conf_thresh, nms_thresh, var0, var1,
+                            out, counts, kept_prior, ws, ws_bytes, stream, 0);
 }
 
 FDT_API int fdt_detect(const float *loc, const float *conf, const float *priors,
@@ -2194,8 +2325,8 @@ FDT_API int fdt_detect(const float *loc, const float *conf, const float *priors,
                        float *out, int32_t *counts, int64_t *kept_prior,
                        void *ws, size_t ws_bytes, fdt_stream_t stream)
 {
-    return fdt_detect_flags(loc, conf, priors, B, N, C, top_k, nms_top_k, conf_thresh, nms_thresh, var0, var1, out, counts, kept_prior,
-                            ws, ws_bytes, stream, 0);
+    return fdt_detect_ex(loc, FDT_DTYPE_F32, conf, FDT_DTYPE_F32, priors, B, N, C, top_k, nms_top_k, conf_thresh, nms_thresh, var0, var1,
+                         out, counts, kept_prior, ws, ws_bytes, stream);
 }
 
 // ---- head maps -> Detect (SURVEY 8f rank 1; pyramid.py:291-309, 331-338)

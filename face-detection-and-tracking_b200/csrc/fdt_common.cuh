@@ -9,11 +9,14 @@
 
 void fdt_set_error(const char *fmt, ...);
 
-// library-internal form of fdt_detect (hostctx.cu): `loc` may be a device view of pinned HOST memory that k_sort_nms gathers in place
+// library-internal form of fdt_detect_ex (hostctx.cu): `loc` may be a device view of pinned HOST memory that k_sort_nms gathers in place
 constexpr unsigned FDT_FLAG_LOC_HOST_MAPPED = 1u;
-int fdt_detect_flags(const float *loc, const float *conf, const float *priors, int B, int64_t N, int C, int top_k, int nms_top_k,
-                     float conf_thresh, float nms_thresh, float var0, float var1, float *out, int32_t *counts, int64_t *kept_prior,
-                     void *ws, size_t ws_bytes, void *stream, unsigned flags);
+int fdt_detect_flags(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *priors, int B, int64_t N, int C,
+                     int top_k, int nms_top_k, float conf_thresh, float nms_thresh, float var0, float var1, float *out, int32_t *counts,
+                     int64_t *kept_prior, void *ws, size_t ws_bytes, void *stream, unsigned flags);
+// the `_ex` entries' checks of flat loc[B,N,4] / conf[B,N,C] (detect.cu): known FDT_DTYPE_*, each pointer aligned to its elements, an
+// fp32 loc to f32_loc_align bytes (16 where the kernels read it as float4 rows; 4 for a host buffer the call copies when it is not)
+int fdt_flat_inputs_ok(const char *who, const void *loc, int loc_dtype, const void *conf, int conf_dtype, size_t f32_loc_align);
 
 constexpr int FDT_DETECT_MAX_DEPTH = 4;     // slots of the stateful Detect workspace (calls of one stream in flight)
 int fdt_option_host_chunk();     // images per copy/compute chunk of the host-buffer pipeline (hostctx.cu); option "host_chunk"

@@ -39,7 +39,8 @@ HostPlan make_plan(int Bc, int64_t N, int C, int top_k)
 {
     HostPlan p;
     p.Bc = Bc; p.C = C; p.top_k = top_k; p.N = N;
-    // per slot: a single-slot Detect workspace (the Bc geometry also holds the remainder chunk's), then the staging buffers
+    // per slot: a single-slot Detect workspace (the Bc geometry also holds the remainder chunk's), then the staging buffers, sized for
+    // fp32 inputs so that one layout serves every element type (a 16-bit conf / loc chunk fills the first half of its buffer)
     p.ws_bytes = fdt_align256(fdt_detect_workspace_bytes_depth(Bc, N, C, 1));
     size_t o = p.ws_bytes;
     p.so_conf = o; o += fdt_align256((size_t)Bc * N * C * 4);
@@ -52,15 +53,15 @@ HostPlan make_plan(int Bc, int64_t N, int C, int top_k)
     return p;
 }
 
-// device view of a pinned (mapped) host pointer, or null
+// device view of a pinned (mapped) host pointer whose device address is `align`-byte aligned, or null
 template <typename T>
-T *mapped_view(T *host)
+T *mapped_view(T *host, size_t align = 16)
 {
     if (!host) return nullptr;
     cudaPointerAttributes attr;
     cudaError_t e = cudaPointerGetAttributes(&attr, (const void *)host);
     if (e != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }   // pageable memory on old drivers reports an error: ignore
-    if (attr.type == cudaMemoryTypeHost && attr.devicePointer && fdt_aligned(attr.devicePointer, 16)) return (T *)attr.devicePointer;
+    if (attr.type == cudaMemoryTypeHost && attr.devicePointer && fdt_aligned(attr.devicePointer, align)) return (T *)attr.devicePointer;
     return nullptr;
 }
 }  // namespace
@@ -194,13 +195,17 @@ FDT_API int fdt_ctx_set_priors(fdt_ctx *c, const float *priors_h, int64_t N)
     return FDT_OK;
 }
 
-FDT_API int fdt_detect_host_submit(fdt_ctx *c, const float *loc_h, const float *conf_h, const float *priors_h,
-                                   int B, int64_t N, int C, int top_k, int nms_top_k,
-                                   float conf_thresh, float nms_thresh, float var0, float var1,
-                                   float *out_h, int32_t *counts_h, int64_t *kept_prior_h, uint64_t *ticket)
+FDT_API int fdt_detect_host_submit_ex(fdt_ctx *c, const void *loc_h, int loc_dtype, const void *conf_h, int conf_dtype,
+                                      const float *priors_h, int B, int64_t N, int C, int top_k, int nms_top_k,
+                                      float conf_thresh, float nms_thresh, float var0, float var1,
+                                      float *out_h, int32_t *counts_h, int64_t *kept_prior_h, uint64_t *ticket)
 {
     FDT_REQUIRE(c != nullptr && ticket != nullptr, FDT_E_INVALID, "fdt_detect_host_submit: null context / ticket");
     FDT_REQUIRE(B >= 0 && N >= 0 && C >= 1 && top_k >= 1, FDT_E_INVALID, "fdt_detect_host_submit: bad sizes");
+    // host buffers: element alignment only -- a loc_h that is not a 16-byte (fp32) / 8-byte (16-bit) aligned pinned buffer is copied
+    int rc = fdt_flat_inputs_ok("fdt_detect_host_submit", loc_h, loc_dtype, conf_h, conf_dtype, 4);
+    if (rc != FDT_OK) return rc;
+    const size_t le = loc_dtype == FDT_DTYPE_F32 ? 4 : 2, ce = conf_dtype == FDT_DTYPE_F32 ? 4 : 2;      // element sizes
     FDT_CUDA(cudaSetDevice(c->device));
     if (B == 0) {                                                          // nothing to do: completes with the previous call
         FDT_CUDA(cudaEventRecord(c->call_done[c->calls % HOST_CALLS], c->stream));
@@ -210,9 +215,8 @@ FDT_API int fdt_detect_host_submit(fdt_ctx *c, const float *loc_h, const float *
     FDT_REQUIRE(loc_h && conf_h && out_h, FDT_E_INVALID, "fdt_detect_host_submit: null pointer argument");
     FDT_REQUIRE(priors_h || c->pri_n == N, FDT_E_INVALID,
                 "fdt_detect_host_submit: priors_h is null and the context holds %lld priors, not %lld", (long long)c->pri_n, (long long)N);
-    int rc;
     if (priors_h && (rc = fdt_ctx_set_priors(c, priors_h, N)) != FDT_OK) return rc;
-    const float *loc_view = mapped_view(loc_h);
+    const char *loc_view = mapped_view((const char *)loc_h, 4 * le);
     float *out_view = mapped_view(out_h);
 
     int chunk = fdt_option_host_chunk();
@@ -226,22 +230,25 @@ FDT_API int fdt_detect_host_submit(fdt_ctx *c, const float *loc_h, const float *
         const int b0 = i * Bc, nb = (i == nchunks - 1 && Br) ? Br : Bc;
         HostSlot &s = c->slot[c->chunks % HOST_SLOTS];
         char *base = (char *)c->buf + (c->chunks % HOST_SLOTS) * p.slot_stride;
-        float *d_conf = (float *)(base + p.so_conf);
-        float *d_locs = (float *)(base + p.so_loc);
+        char *d_conf = base + p.so_conf;
+        char *d_locs = base + p.so_loc;
         float *d_outs = (float *)(base + p.so_out);
         int32_t *d_cnt = (int32_t *)(base + p.so_cnt);
         int64_t *d_kept = (int64_t *)(base + p.so_kept);
         if (s.used) FDT_CUDA(cudaStreamWaitEvent(c->copy, s.done, 0));     // the slot's previous chunk has been consumed
-        FDT_CUDA(cudaMemcpyAsync(d_conf, conf_h + (size_t)b0 * N * C, (size_t)nb * N * C * 4, cudaMemcpyHostToDevice, c->copy));
-        if (!loc_view) FDT_CUDA(cudaMemcpyAsync(d_locs, loc_h + (size_t)b0 * N * 4, (size_t)nb * N * 16, cudaMemcpyHostToDevice, c->copy));
+        FDT_CUDA(cudaMemcpyAsync(d_conf, (const char *)conf_h + (size_t)b0 * N * C * ce, (size_t)nb * N * C * ce, cudaMemcpyHostToDevice,
+                                 c->copy));
+        if (!loc_view)
+            FDT_CUDA(cudaMemcpyAsync(d_locs, (const char *)loc_h + (size_t)b0 * N * 4 * le, (size_t)nb * N * 4 * le, cudaMemcpyHostToDevice,
+                                     c->copy));
         FDT_CUDA(cudaEventRecord(s.copied, c->copy));                      // (behind the prior upload, if this call made one)
         FDT_CUDA(cudaStreamWaitEvent(s.st, s.copied, 0));
         // rows in place only where the chunk's block is 16-byte aligned in the caller's buffer
         float *o_view = out_view ? out_view + (size_t)b0 * row_out * 5 : nullptr;
         if (o_view && !fdt_aligned(o_view, 16)) o_view = nullptr;
-        rc = fdt_detect_flags(loc_view ? loc_view + (size_t)b0 * N * 4 : d_locs, d_conf, d_pri, nb, N, C, top_k, nms_top_k, conf_thresh,
-                              nms_thresh, var0, var1, o_view ? o_view : d_outs, counts_h ? d_cnt : nullptr, kept_prior_h ? d_kept : nullptr,
-                              base, p.ws_bytes, s.st, loc_view ? FDT_FLAG_LOC_HOST_MAPPED : 0u);
+        rc = fdt_detect_flags(loc_view ? loc_view + (size_t)b0 * N * 4 * le : d_locs, loc_dtype, d_conf, conf_dtype, d_pri, nb, N, C, top_k,
+                              nms_top_k, conf_thresh, nms_thresh, var0, var1, o_view ? o_view : d_outs, counts_h ? d_cnt : nullptr,
+                              kept_prior_h ? d_kept : nullptr, base, p.ws_bytes, s.st, loc_view ? FDT_FLAG_LOC_HOST_MAPPED : 0u);
         if (rc != FDT_OK) return rc;
         if (!o_view)
             FDT_CUDA(cudaMemcpyAsync(out_h + (size_t)b0 * row_out * 5, d_outs, (size_t)nb * row_out * 20, cudaMemcpyDeviceToHost, s.st));
@@ -270,14 +277,32 @@ FDT_API int fdt_detect_host_wait(fdt_ctx *c, uint64_t ticket)
     return FDT_OK;
 }
 
+FDT_API int fdt_detect_host_submit(fdt_ctx *c, const float *loc_h, const float *conf_h, const float *priors_h,
+                                   int B, int64_t N, int C, int top_k, int nms_top_k,
+                                   float conf_thresh, float nms_thresh, float var0, float var1,
+                                   float *out_h, int32_t *counts_h, int64_t *kept_prior_h, uint64_t *ticket)
+{
+    return fdt_detect_host_submit_ex(c, loc_h, FDT_DTYPE_F32, conf_h, FDT_DTYPE_F32, priors_h, B, N, C, top_k, nms_top_k, conf_thresh,
+                                     nms_thresh, var0, var1, out_h, counts_h, kept_prior_h, ticket);
+}
+
+FDT_API int fdt_detect_host_ex(fdt_ctx *c, const void *loc_h, int loc_dtype, const void *conf_h, int conf_dtype, const float *priors_h,
+                               int B, int64_t N, int C, int top_k, int nms_top_k,
+                               float conf_thresh, float nms_thresh, float var0, float var1,
+                               float *out_h, int32_t *counts_h, int64_t *kept_prior_h)
+{
+    uint64_t t = 0;
+    int rc = fdt_detect_host_submit_ex(c, loc_h, loc_dtype, conf_h, conf_dtype, priors_h, B, N, C, top_k, nms_top_k, conf_thresh,
+                                       nms_thresh, var0, var1, out_h, counts_h, kept_prior_h, &t);
+    if (rc != FDT_OK) return rc;
+    return fdt_detect_host_wait(c, t);
+}
+
 FDT_API int fdt_detect_host(fdt_ctx *c, const float *loc_h, const float *conf_h, const float *priors_h,
                             int B, int64_t N, int C, int top_k, int nms_top_k,
                             float conf_thresh, float nms_thresh, float var0, float var1,
                             float *out_h, int32_t *counts_h, int64_t *kept_prior_h)
 {
-    uint64_t t = 0;
-    int rc = fdt_detect_host_submit(c, loc_h, conf_h, priors_h, B, N, C, top_k, nms_top_k, conf_thresh, nms_thresh, var0, var1,
-                                    out_h, counts_h, kept_prior_h, &t);
-    if (rc != FDT_OK) return rc;
-    return fdt_detect_host_wait(c, t);
+    return fdt_detect_host_ex(c, loc_h, FDT_DTYPE_F32, conf_h, FDT_DTYPE_F32, priors_h, B, N, C, top_k, nms_top_k, conf_thresh,
+                              nms_thresh, var0, var1, out_h, counts_h, kept_prior_h);
 }

@@ -53,7 +53,9 @@ class Detect:
     def __call__(self, loc_data, conf_data, prior_data, return_aux=False):
         """loc_data [B,N,4] (or [B,N*4]), conf_data [B,N,C] (or [B*N,C]) post-softmax, prior_data [N,4]
         -> output [B, num_classes, top_k, 5] rows [score, x1, y1, x2, y2].
-        return_aux=True additionally returns (counts[B,C] int32, kept_prior[B,C,top_k] int64)."""
+        return_aux=True additionally returns (counts[B,C] int32, kept_prior[B,C,top_k] int64).
+        Contiguous bf16 / fp16 loc_data / conf_data (autocast, .half() models) are read in place; the result is bit-identical to the
+        call on loc_data.float(), conf_data.float() (scores compared with conf_thresh in fp32)."""
         _lib.require_cuda()
         num = loc_data.size(0)
         num_priors = prior_data.size(0)
@@ -64,16 +66,17 @@ class Detect:
             return self._call_host(loc_data, conf_data, prior_data, args, return_aux)
         dev = loc_data.device
         with torch.cuda.device(dev):
-            loc = _lib.dev_f32(loc_data, dev).view(num, num_priors, 4)
-            conf = _lib.dev_f32(conf_data, dev).view(num, num_priors, C_)
+            loc, ldt = _lib.flat_input(loc_data, dev)
+            conf, cdt = _lib.flat_input(conf_data, dev)
+            loc, conf = loc.view(num, num_priors, 4), conf.view(num, num_priors, C_)
             pri = _lib.dev_f32(prior_data, dev).view(num_priors, 4)
             out = torch.empty((num, C_, self.top_k, 5), dtype=torch.float32, device=dev)
             counts = torch.empty((num, C_), dtype=torch.int32, device=dev) if return_aux else None
             kept = torch.empty((num, C_, self.top_k), dtype=torch.int64, device=dev) if return_aux else None
             L = _lib.lib()
             ws = self._workspaces.get(num, num_priors, C_, dev)
-            _lib.check(L.fdt_detect(_lib.ptr(loc), _lib.ptr(conf), _lib.ptr(pri), *args, _lib.ptr(out),
-                                    _lib.ptr(counts), _lib.ptr(kept), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
+            _lib.check(L.fdt_detect_ex(_lib.ptr(loc), ldt, _lib.ptr(conf), cdt, _lib.ptr(pri), *args, _lib.ptr(out),
+                                       _lib.ptr(counts), _lib.ptr(kept), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
         return (out, counts, kept) if return_aux else out
 
     def detect_heads(self, loc_maps, conf_maps, prior_data, neg_max=None, return_aux=False):
@@ -110,15 +113,16 @@ class Detect:
         (fdt_detect_host_submit) and returns a PendingDetections whose .result() blocks until the output landed.  Keeping two
         batches in flight hides everything but the host-to-device copy of `conf`.  Pinned inputs make the submit non-blocking;
         the tensors must stay untouched until .result().  A prior tensor that was already uploaded by this thread (same storage,
-        same version counter) is not copied again."""
+        same version counter) is not copied again.  Contiguous bf16 / fp16 inputs cross the link at their own size."""
         _lib.require_cuda()
         if loc_data.is_cuda:
             raise ValueError("Detect.submit is the host-tensor path; CUDA tensors are already asynchronous through __call__")
         num, num_priors, C_ = loc_data.size(0), prior_data.size(0), self.num_classes
         args = (num, num_priors, C_, int(self.top_k), int(self.nms_top_k), float(self.conf_thresh),
                 float(self.nms_thresh), float(self.variance[0]), float(self.variance[1]))
-        loc = loc_data.detach().to(torch.float32).contiguous()
-        conf = conf_data.detach().to(torch.float32).contiguous()
+        host = torch.device("cpu")
+        loc, ldt = _lib.flat_input(loc_data, host)
+        conf, cdt = _lib.flat_input(conf_data, host)
         pri = prior_data.detach().to(torch.float32).contiguous().cpu()
         out = torch.empty((num, C_, self.top_k, 5), dtype=torch.float32, pin_memory=True)
         counts = torch.empty((num, C_), dtype=torch.int32, pin_memory=True) if return_aux else None
@@ -131,8 +135,8 @@ class Detect:
         key = (pri.data_ptr(), pri._version, num_priors)
         hit = dev_index in resident and resident[dev_index][0] == key
         ticket = C.c_uint64(0)
-        _lib.check(_lib.lib().fdt_detect_host_submit(ctx, _lib.ptr(loc), _lib.ptr(conf), None if hit else _lib.ptr(pri),
-                                                     *args, _lib.ptr(out), _lib.ptr(counts), _lib.ptr(kept), C.byref(ticket)))
+        _lib.check(_lib.lib().fdt_detect_host_submit_ex(ctx, _lib.ptr(loc), ldt, _lib.ptr(conf), cdt, None if hit else _lib.ptr(pri),
+                                                        *args, _lib.ptr(out), _lib.ptr(counts), _lib.ptr(kept), C.byref(ticket)))
         resident[dev_index] = (key, pri)
         return PendingDetections(ctx, ticket.value, (out, counts, kept) if return_aux else out, (loc, conf, pri))
 

@@ -35,8 +35,8 @@ class _MultiBoxLossFn(torch.autograd.Function):
         dev = loc_data.device
         B, N, _ = loc_data.shape
         C_ = conf_data.shape[-1]
-        loc = _lib.dev_f32(loc_data, dev)
-        conf = _lib.dev_f32(conf_data, dev)
+        loc, ldt = _lib.flat_input(loc_data, dev)           # bf16 / fp16 in place (autocast), anything else as fp32
+        conf, cdt = _lib.flat_input(conf_data, dev)
         pri = _lib.dev_f32(priors, dev)
         losses = torch.empty(2, dtype=torch.float32, device=dev)
         norm = torch.empty(1, dtype=torch.float32, device=dev)
@@ -46,12 +46,13 @@ class _MultiBoxLossFn(torch.autograd.Function):
         with torch.cuda.device(dev):
             L = _lib.lib()
             ws = _lib.workspace(L.fdt_multibox_workspace_bytes(B, N, C_, total_gt), dev, "multibox")
-            _lib.check(L.fdt_multibox_loss_forward(
-                _lib.ptr(loc), _lib.ptr(conf), _lib.ptr(pri), _lib.ptr(gt), _lib.ptr(gt_off), total_gt, B, N, C_,
+            _lib.check(L.fdt_multibox_loss_forward_ex(
+                _lib.ptr(loc), ldt, _lib.ptr(conf), cdt, _lib.ptr(pri), _lib.ptr(gt), _lib.ptr(gt_off), total_gt, B, N, C_,
                 float(threshold), int(negpos_ratio), int(bool(bipartite)), float(variance[0]), float(variance[1]),
                 _lib.ptr(losses), _lib.ptr(norm), _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), None,
                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr()))
         ctx.save_for_backward(loc, conf, loc_t, conf_t, sel, norm)
+        ctx.dtypes = (ldt, cdt)
         ctx.mark_non_differentiable(loc_t, conf_t, sel)
         # two independent 0-dim tensors, as the reference returns (views of one buffer would forbid in-place ops on them)
         return losses[0].clone(), losses[1].clone(), loc_t, conf_t, sel
@@ -61,7 +62,7 @@ class _MultiBoxLossFn(torch.autograd.Function):
         loc, conf, loc_t, conf_t, sel, norm = ctx.saved_tensors
         B, N, _ = loc.shape
         C_ = conf.shape[-1]
-        grad_loc = torch.empty_like(loc)
+        grad_loc = torch.empty_like(loc)                    # in the dtypes of what the kernels read (the fp32 gradients rounded)
         grad_conf = torch.empty_like(conf)
         # the upstream gradients stay on the device: no float() synchronisation, the loss can be captured in a CUDA graph
         dev = loc.device
@@ -75,8 +76,8 @@ class _MultiBoxLossFn(torch.autograd.Function):
             return g.detach().to(device=dev, dtype=torch.float32).contiguous()
         gl, gc = scalar(g_l), scalar(g_c)
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().fdt_multibox_loss_backward_dev(
-                _lib.ptr(loc), _lib.ptr(conf), _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), _lib.ptr(norm),
+            _lib.check(_lib.lib().fdt_multibox_loss_backward_dev_ex(
+                _lib.ptr(loc), ctx.dtypes[0], _lib.ptr(conf), ctx.dtypes[1], _lib.ptr(loc_t), _lib.ptr(conf_t), _lib.ptr(sel), _lib.ptr(norm),
                 _lib.ptr(gl), _lib.ptr(gc), B, N, C_, _lib.ptr(grad_loc), _lib.ptr(grad_conf), _lib.stream_ptr()))
         return grad_loc, grad_conf, None, None, None, None, None, None, None, None
 

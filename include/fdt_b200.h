@@ -159,6 +159,17 @@ int fdt_detect(const float *loc, const float *conf, const float *priors,
                float conf_thresh, float nms_thresh, float var0, float var1,
                float *out, int32_t *counts, int64_t *kept_prior,
                void *ws, size_t ws_bytes, fdt_stream_t stream);
+/* Mixed precision (what a model under torch.autocast, or one converted with .half() / .to(torch.bfloat16), hands over): loc and conf
+ * each of element type loc_dtype / conf_dtype (FDT_DTYPE_F32 / _BF16 / _F16, defined below), read in place.  Every element is widened
+ * to fp32 exactly and all arithmetic is what it is on fp32 inputs, so out / counts / kept_prior are bit-identical to fdt_detect on the
+ * inputs converted to fp32.  The threshold is compared in fp32 against the widened score (score > conf_thresh), not rounded to the
+ * input's type first.  Each pointer must be aligned to its element size, an fp32 loc to 16 bytes; an unknown dtype or a misaligned
+ * pointer is FDT_E_INVALID before any CUDA call.  fdt_detect == fdt_detect_ex with two FDT_DTYPE_F32. */
+int fdt_detect_ex(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *priors,
+                  int B, int64_t N, int C, int top_k, int nms_top_k,
+                  float conf_thresh, float nms_thresh, float var0, float var1,
+                  float *out, int32_t *counts, int64_t *kept_prior,
+                  void *ws, size_t ws_bytes, fdt_stream_t stream);
 /* Overlap of consecutive calls.  A workspace of fdt_detect_workspace_bytes_depth(B, N, C, depth) bytes, depth 2..4, holds `depth`
  * slots of per-call scratch: call s uses slot s % depth, so the threshold pass of call s + 1 runs while the NMS kernel of call s is
  * still in flight and its NMS CTAs take over SMs as those of call s retire (all on ONE stream, chained by programmatic dependent
@@ -297,6 +308,18 @@ int fdt_detect_host_submit(fdt_ctx *ctx, const float *loc_h, const float *conf_h
                            float conf_thresh, float nms_thresh, float var0, float var1,
                            float *out_h, int32_t *counts_h, int64_t *kept_prior_h, uint64_t *ticket);
 int fdt_detect_host_wait(fdt_ctx *ctx, uint64_t ticket);
+/* the same on bf16 / fp16 / fp32 host tensors (as fdt_detect_ex): conf chunks cross the link at their own element size, a pinned loc_h
+ * is gathered in place (8-byte aligned 16-bit rows, 16-byte fp32 rows), any other is copied at its own size.  Host buffers need only be
+ * aligned to their elements.  One context serves every
+ * dtype.  fdt_detect_host / _submit == these with two FDT_DTYPE_F32. */
+int fdt_detect_host_ex(fdt_ctx *ctx, const void *loc_h, int loc_dtype, const void *conf_h, int conf_dtype, const float *priors_h,
+                       int B, int64_t N, int C, int top_k, int nms_top_k,
+                       float conf_thresh, float nms_thresh, float var0, float var1,
+                       float *out_h, int32_t *counts_h, int64_t *kept_prior_h);
+int fdt_detect_host_submit_ex(fdt_ctx *ctx, const void *loc_h, int loc_dtype, const void *conf_h, int conf_dtype, const float *priors_h,
+                              int B, int64_t N, int C, int top_k, int nms_top_k,
+                              float conf_thresh, float nms_thresh, float var0, float var1,
+                              float *out_h, int32_t *counts_h, int64_t *kept_prior_h, uint64_t *ticket);
 
 /* ---- M4/M5  match_default / match_ensure_max_prior (layers/box_utils.py:165-210, 103-162) -------
  * Batched over images: gt[total_gt,5] rows [x1,y1,x2,y2,label], gt_off[B+1] int64 (device).
@@ -339,6 +362,18 @@ int fdt_multibox_loss_backward(const float *loc, const float *conf, const float 
 int fdt_multibox_loss_backward_dev(const float *loc, const float *conf, const float *loc_t, const int64_t *conf_t,
                                    const uint8_t *sel, const float *norm, const float *g_l_dev, const float *g_c_dev,
                                    int B, int64_t N, int C, float *grad_loc, float *grad_conf, fdt_stream_t stream);
+/* Mixed precision: loc / conf of element types loc_dtype / conf_dtype (FDT_DTYPE_*), read in place, each pointer aligned to its element
+ * size (an fp32 loc to 16 bytes; the forward's fp32 conf with C == 2 to 8, as before); the outputs are bit-identical to the entries above on the inputs
+ * converted to fp32.  grad_loc / grad_conf have the element types of loc / conf: the fp32 gradients rounded to nearest even.  An
+ * unknown dtype or a misaligned pointer is FDT_E_INVALID before any CUDA call.  The entries above are these with FDT_DTYPE_F32. */
+int fdt_multibox_loss_forward_ex(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *priors,
+                                 const float *gt, const int64_t *gt_off, int64_t total_gt, int B, int64_t N, int C,
+                                 float threshold, int negpos_ratio, int bipartite, float var0, float var1,
+                                 float *losses, float *norm, float *loc_t, int64_t *conf_t, uint8_t *sel,
+                                 float *loss_c_all, void *ws, size_t ws_bytes, fdt_stream_t stream);
+int fdt_multibox_loss_backward_dev_ex(const void *loc, int loc_dtype, const void *conf, int conf_dtype, const float *loc_t,
+                                      const int64_t *conf_t, const uint8_t *sel, const float *norm, const float *g_l_dev,
+                                      const float *g_c_dev, int B, int64_t N, int C, void *grad_loc, void *grad_conf, fdt_stream_t stream);
 
 /* ---- training from head maps (SURVEY 8f rank 1; replaces pyramid.py:291-309 + MyTrain_repo.py:170-171 and their autograd backward)
  * Map arguments as fdt_heads_to_loc_conf (HOST arrays of n_levels DEVICE pointers, NCHW [B,4,H_l,W_l]; the `_ex` entries: HOST arrays
