@@ -22,6 +22,7 @@
 //
 // Tie rule (unspecified in the reference, torch.sort is unstable): keys are unique, descending key order = descending score,
 // higher prior index first among equal scores.  DESIGN.md section 4 has the exactness arguments.
+#include <algorithm>
 #include <atomic>
 #include <cstdlib>
 #include <mutex>
@@ -968,6 +969,32 @@ k_sort_nms(const SortNmsParams P)
     const float *crow = FUSED ? P.conf + ((int64_t)b * P.N) * P.C + cl : nullptr;
     const float cthr = P.conf_thresh;
     const int n_scan = FUSED ? (int)P.N : n_c;               // entries a full pass looks at
+    // FUSED: the windows usually stop long before nms_top_k (the headline keeps its 750 boxes within the first ~900 of 5,000 candidates),
+    // so stage 1 selects and scatters the k_all = min(candidates, nms_top_k) best keys in chunks of at most two first windows.  When the
+    // windows have consumed a chunk without reaching max_keep, the next chunk is selected the same way among the keys below `tmax`, the
+    // last key processed, by a re-scan of the row in place (the queues are window arrays by then).  Chunks follow score order, so the
+    // windows see exactly the sequence of the unchunked selection.  What the windows carry from one chunk to the next waits in shared
+    // memory (`s_ck`), so that none of it occupies registers during stage 1.
+    struct ChunkState {
+        uint64_t tmax;                                       // only keys below it take part (later chunks)
+        int chunk, k_all, done_k;                            // chunk number, min(candidates, nms_top_k), candidates of earlier chunks
+        int nkept, rounds, sweeps, win_cap;
+        GridGeom gg;
+    };
+    __shared__ ChunkState s_ck;
+    if (tid == 0) {
+        s_ck.tmax = ~0ull; s_ck.chunk = 0; s_ck.k_all = k; s_ck.done_k = 0;
+        s_ck.nkept = 0; s_ck.rounds = 0; s_ck.sweeps = 0;
+        // Window size.  Detect stops at max_keep kept boxes, so a window only needs the candidates that get it there: the first one takes
+        // 1.2 x max_keep (+16) of them, later ones what the keep rate of the previous window predicts (+1/8 + 32) -- at least one whole
+        // bucket more than the largest bucket of the range (BIG_BUCKET), at most WIN.  Windows are consumed in score order whatever their
+        // size, so the result does not depend on it; a short window leaves warps idle in every phase of the round.
+        s_ck.win_cap = MODE == MODE_DETECT ? min(WIN, max(BIG_BUCKET + 64, (P.max_keep * 6) / 5 + 16)) : WIN;
+        s_ck.gg.ok = 0; s_ck.gg.x0 = s_ck.gg.y0 = s_ck.gg.inv0 = s_ck.gg.c0 = 0.0f;
+    }
+    int nkept_out = 0, rounds_out = 0, sweeps_out = 0;
+    for (;;) {
+    presorted = false;
     if (FUSED || k > 0) {
         constexpr int KREG = FUSED ? 1 : 8;
         const bool cached = !FUSED && n_c <= KREG * K3_THREADS;
@@ -1097,7 +1124,10 @@ k_sort_nms(const SortNmsParams P)
                     float sc;
                     if constexpr (HT == 1) sc = conf_any(i);
                     else sc = __ldg(crow + (int64_t)i * Cc);
-                    if (sc > cthr) body(key_of(sc, i));
+                    if (sc > cthr) {
+                        const uint64_t kq = key_of(sc, i);
+                        if (!FUSED || kq < s_ck.tmax) body(kq);
+                    }
                 }
             } else if (cached) {
 #pragma unroll
@@ -1109,6 +1139,7 @@ k_sort_nms(const SortNmsParams P)
         if (tid == 0) { s_kmin = 0xffffffffu; s_kmax = 0u; s_maxb = 0; }
         for (int i = tid; i < 2 * NB; i += K3_THREADS) s_hist[i] = 0;
         __syncthreads();
+        if (FUSED && s_ck.chunk > 0) { scanned = true; wq_ovf = true; }      // (uniform) the queues are gone: in place
         unsigned kmax;
         if (FUSED) {
             // the score range is known beforehand: every candidate is above conf_thresh, softmax outputs end at 1.  Anything beyond
@@ -1153,9 +1184,15 @@ k_sort_nms(const SortNmsParams P)
             }
             __syncthreads();
             if (FUSED && attempt == 0) {                         // the first row scan counted the candidates
-                n_c = s_warp[32];
-                if (MODE == MODE_DETECT && n_c == 1) n_c = 0;    // detection.py:66-72: one candidate -> `continue`
-                k = min(n_c, P.nms_top_k);
+                if (s_ck.chunk == 0) {
+                    n_c = s_warp[32];
+                    if (MODE == MODE_DETECT && n_c == 1) n_c = 0;    // detection.py:66-72: one candidate -> `continue`
+                    k = min(n_c, P.nms_top_k);
+                    if (tid == 0) s_ck.k_all = k;                // (read after the windows' barriers only)
+                } else {
+                    k = s_ck.k_all - s_ck.done_k;
+                }
+                k = min(k, 2 * s_ck.win_cap);
                 if (k == 0) break;                               // (uniform)
             }
             int run = inc - sum + s_warp[warp], mb = 0;
@@ -1188,8 +1225,8 @@ k_sort_nms(const SortNmsParams P)
                             float sc;
                             if constexpr (HT == 1) sc = conf_any(i);
                             else sc = __ldg(crow + (int64_t)i * P.C);
-                            cand = sc > cthr;
                             key = ((uint64_t)fdt_float_key(sc) << 32) | (uint32_t)i;
+                            cand = sc > cthr && key < s_ck.tmax;
                         } else key = __ldcg(gkeys + i);
                         if (cand && (key & pmask) == prefix) d = (int)((key >> shift) & 0xff);
                     }
@@ -1265,6 +1302,8 @@ k_sort_nms(const SortNmsParams P)
         }
         }
         K3_STAMP(2);
+    } else {
+        __syncthreads();                                     // (no candidates, not fused) publishes s_ck
     }
 
     // =========================================================== stage 2: lazy greedy NMS over windows of sorted candidates
@@ -1290,16 +1329,9 @@ k_sort_nms(const SortNmsParams P)
         return fdt_suppresses(bi, ai, bj2, aj2, thr);
     };
     const int max_keep = P.max_keep;
-    int nkept = 0, rounds = 0, sweeps = 0;
-    GridGeom gg;
-    gg.ok = 0; gg.x0 = gg.y0 = gg.inv0 = gg.c0 = 0.0f;
-
-    // Window size.  Detect stops at max_keep kept boxes, so a window only needs the candidates that get it there: the first one takes
-    // 1.2 x max_keep (+16) of them, later ones what the keep rate of the previous window predicts (+1/8 + 32) -- at least one whole
-    // bucket more than the largest bucket of the range (BIG_BUCKET), at most WIN.  Windows are consumed in score order whatever their
-    // size, so the result does not depend on it; a short window leaves warps idle in every phase of the round.
-    int win_cap = WIN;
-    if (MODE == MODE_DETECT) win_cap = min(WIN, max(BIG_BUCKET + 64, (max_keep * 6) / 5 + 16));
+    int nkept = s_ck.nkept, rounds = s_ck.rounds, sweeps = s_ck.sweeps;        // (s_ck: see stage 1)
+    GridGeom gg = s_ck.gg;
+    int win_cap = s_ck.win_cap;
     for (int lo = 0; lo < k && nkept < max_keep; ++rounds) {
         // ---- window [lo, hi): whole buckets, at most win_cap candidates
         int hi;
@@ -1604,6 +1636,18 @@ k_sort_nms(const SortNmsParams P)
         K3_ACC(6);
         lo = hi;
     }
+    nkept_out = nkept; rounds_out = rounds; sweeps_out = sweeps;
+    if (!FUSED || nkept >= max_keep || s_ck.done_k + k >= s_ck.k_all) break;      // (uniform)
+    // next chunk: the last key of this one is in exact order (its window ranked it); once every thread has evaluated the test above,
+    // thread 0 records the state, and the first barrier of stage 1 publishes it
+    __syncthreads();
+    if (tid == 0) {
+        s_ck.tmax = skeys[k - 1]; s_ck.done_k += k; s_ck.chunk += 1;
+        s_ck.nkept = nkept; s_ck.rounds = rounds; s_ck.sweeps = sweeps; s_ck.win_cap = win_cap; s_ck.gg = gg;
+    }
+    }
+    const int nkept = nkept_out, rounds = rounds_out, sweeps = sweeps_out;
+    if (FUSED) k = s_ck.k_all;
     if (prof) {
         for (int q = 0; q < 6; ++q) atomicAdd((unsigned long long *)&P.prof[5 + q], (unsigned long long)pacc[q]);
         atomicAdd((unsigned long long *)&P.prof[16], (unsigned long long)pacc[6]);
@@ -1833,9 +1877,12 @@ int launch_sort_nms(SortNmsParams &P, int lists, int kcap, void *kept_ws, size_t
     }
     FDT_REQUIRE(kcap <= FDT_MAX_NMS_TOP_K, FDT_E_UNSUPPORTED, "nms_top_k=%d exceeds %d", kcap, FDT_MAX_NMS_TOP_K);
     const int limit = FDT_SMEM_MAX - K3_STATIC_SMEM;
-    SmemPlan sp = plan_smem(kcap, P.max_keep, true);
+    const bool fused = MODE == MODE_DETECT && P.conf != nullptr;
+    // the fused kernel selects at most two first windows (<= 2 x WIN keys) per chunk: its key array need not hold nms_top_k keys
+    const int kslot = fused ? std::min(kcap, 2 * WIN) : kcap;
+    SmemPlan sp = plan_smem(kslot, P.max_keep, true);
     if (sp.total > limit) {
-        sp = plan_smem(kcap, P.max_keep, false);
+        sp = plan_smem(kslot, P.max_keep, false);
         const size_t need = (size_t)lists * P.max_keep * KEPT_ROW_BYTES;
         FDT_REQUIRE(kept_ws_bytes >= need && (kept_ws != nullptr || P.S.ctl != nullptr), FDT_E_WORKSPACE,
                     "kept rows (%d per list) do not fit in shared memory and the workspace lacks %zu bytes for them", P.max_keep, need);
@@ -1854,7 +1901,6 @@ int launch_sort_nms(SortNmsParams &P, int lists, int kcap, void *kept_ws, size_t
     // counts: the cluster repeats every stage but phase B in both CTAs, so it is only used when the workspace has a single slot.
     // Kept rows in global memory (large max_keep) stay on the single-CTA path.
     const int want = opt.k3_cluster.load();
-    const bool fused = MODE == MODE_DETECT && P.conf != nullptr;
     const bool fits = lists * 2 <= FDT_NUM_SMS && sp.off_kbox >= 0;
     const bool cluster = !fused && fits && (want < 0 ? (P.S.ctl == nullptr || P.S.depth == 1) : want == 1);
     const bool pdl = opt.k3_pdl.load() == 1;
